@@ -218,6 +218,7 @@ def test_vip_set_over_http_changes_dispatch_order_like_the_reference():
             s.d.set_online(b, False)                                  # queue everything first (the t=0 arrival trace)
         assert _admin(s, "/admin/vip", {"user": "charlie"})[0] == 200
         streams = [s.d.submit(u, max_new_tokens=1) for u in users for _ in range(8)]
+        s.d.wait_parked()    # the submits' wake-ups are handled: no dispatch can start with only backend 0 back online
         for b in range(2):
             s.d.set_online(b, True)
         s.d.submit("zz-wake", max_new_tokens=1)                       # a notify wakes the scheduler (recovery does not)
