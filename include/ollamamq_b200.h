@@ -150,6 +150,9 @@ int mq_worker_healthy(mq_worker* w);
 #define MQ_EP_V1_CHAT 2        /* /v1/chat/completions     SSE    */
 #define MQ_EP_V1_COMPLETIONS 3 /* /v1/completions          SSE    */
 #define MQ_EP_RAW_TOKENS 4     /* no framing: chunks are little-endian int32 token ids                    */
+/* Raw-token record of a request with logprobs on (mq_request.logprobs != 0, N = top_logprobs): one chunk per token is
+ * int32 id, float32 logprob, then N x (int32 id, float32 logprob), little-endian (8 + 8 N bytes); with logprobs off it
+ * stays the 4-byte id.  stream = 0 concatenates the same records.                                                  */
 #define MQ_EP_EMBED 6          /* /api/embed, /api/embeddings, /v1/embeddings: one JSON reply, served by the
                                   embedding worker attached to the backend (section 2b); `path` picks the
                                   reply shape; 501 when no encoder is attached                             */
@@ -178,8 +181,21 @@ typedef struct mq_request {
   int32_t body_kind;         /* MQ_BODY_JSON: `body` is the client's JSON.  MQ_BODY_TEXT: the front already parsed
                               * it (on its connection thread, never on the scheduler's) and `body` is the extracted
                               * prompt text; stream / max_new_tokens / sampling fields above carry the rest       */
-  int32_t reserved;
+  /* token log-probabilities (0 = off, so a zeroed struct asks for none).  logprobs != 0: every relayed token carries
+   * its logprob and the top_logprobs (clamped to 0..MQ_TOP_LOGPROBS_MAX) most probable tokens with theirs.  Defined
+   * as log-softmax of the raw logits the token was drawn from (temperature 1, before top-k / top-p), alternatives
+   * ordered by logit descending then token id ascending; the EOS token that ends a generation gets no entry.  A JSON
+   * body may carry them too ("logprobs": true / false and "top_logprobs": N; on /v1/completions the legacy
+   * "logprobs": N) and wins over these fields.  Turning them on never changes a token.                        */
+  int16_t logprobs;
+  int16_t top_logprobs;
 } mq_request;
+#define MQ_TOP_LOGPROBS_MAX 20
+#ifdef __cplusplus
+static_assert(sizeof(mq_request) == 88, "mq_request layout is part of the ABI");
+#else
+_Static_assert(sizeof(mq_request) == 88, "mq_request layout is part of the ABI");
+#endif
 #define MQ_BODY_JSON 0
 #define MQ_BODY_TEXT 1
 
@@ -414,9 +430,22 @@ long long mq_debug_frame_embeddings(const char* path, const char* model, const f
                                     int32_t n_tokens, char* out, size_t cap);
 long long mq_debug_frame_final(int32_t endpoint, int32_t stream, const char* model, const char* agg, int32_t n_prompt,
                                int32_t n_gen, int32_t stopped, char* out, size_t cap);
+/* the whole reply of a generation request with n tokens: ids[n], records = n x (float logprob, N x (int32 id, float
+ * logprob)) (the raw-token record without its leading id); top_logprobs < 0 = logprobs off.  stream = 1: the per-token frames then
+ * the final frame, concatenated; stream = 0: the final object.  MQ_EP_RAW_TOKENS: the binary records (length =
+ * return value - 1)                                                                                            */
+long long mq_debug_frame_logprobs(int32_t endpoint, int32_t stream, const char* model, const int32_t* ids,
+                                  const float* records, int32_t n, int32_t top_logprobs, int32_t n_prompt, char* out,
+                                  size_t cap);
 /* the sampler kernel on given logits: per-row controls (device arrays, row == slot), counter = RNG position  */
 int mq_debug_sample(const float* logits, int rows, int V, int ldl, int* out_tokens, const float* temperature,
                     const int* top_k, const float* top_p, const unsigned long long* seed, const int* counter);
+/* the same with log-probability records: top_logprobs = device int[rows] (-1 = no record for that row, 0..20 = that
+ * many alternatives), lp_out = device [rows] records of 164 bytes: float logprob, int32 id[20], float lp[20]
+ * (entries past the row's N and the records of -1 rows are left as they were)                                  */
+int mq_debug_sample_logprobs(const float* logits, int rows, int V, int ldl, int* out_tokens, const float* temperature,
+                             const int* top_k, const float* top_p, const unsigned long long* seed, const int* counter,
+                             const int* top_logprobs, void* lp_out);
 int mq_debug_argmax(const float* logits, int rows, int V, int ldl, int* out_tokens, const int* dst_slot,
                     int* cur_token, int* pos_inc, const int* active);
 int mq_debug_init_normal(void* w, unsigned long long n, unsigned long long seed, float std);

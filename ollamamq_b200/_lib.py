@@ -65,7 +65,10 @@ class Request(C.Structure):
                 ("prompt_tokens", C.c_void_p), ("n_prompt_tokens", C.c_int32), ("max_new_tokens", C.c_int32),
                 ("ignore_eos", C.c_int32), ("timeout_ms", C.c_uint32), ("path", C.c_char_p),
                 ("temperature", C.c_float), ("top_k", C.c_int32), ("top_p", C.c_float), ("seed", C.c_uint64),
-                ("body_kind", C.c_int32), ("reserved", C.c_int32)]
+                ("body_kind", C.c_int32), ("logprobs", C.c_int16), ("top_logprobs", C.c_int16)]
+
+
+MQ_TOP_LOGPROBS_MAX = 20
 
 
 ON_STATUS = C.CFUNCTYPE(None, C.c_void_p, C.c_int32, C.c_char_p)
@@ -212,6 +215,9 @@ _sig("mq_debug_frame_embeddings", C.c_longlong, [C.c_char_p, C.c_char_p, P, C.c_
 _sig("mq_debug_frame_final", C.c_longlong, [C.c_int32, C.c_int32, C.c_char_p, C.c_char_p, C.c_int32, C.c_int32, C.c_int32, P,
                                               C.c_size_t])
 _sig("mq_debug_sample", C.c_int, [P, C.c_int, C.c_int, C.c_int, P, P, P, P, P, P])
+_sig("mq_debug_sample_logprobs", C.c_int, [P, C.c_int, C.c_int, C.c_int, P, P, P, P, P, P, P, P])
+_sig("mq_debug_frame_logprobs", C.c_longlong, [C.c_int32, C.c_int32, C.c_char_p, P, P, C.c_int32, C.c_int32, C.c_int32, P,
+                                                 C.c_size_t])
 _sig("mq_debug_argmax", C.c_int, [P, C.c_int, C.c_int, C.c_int, P, P, P, P, P])
 _sig("mq_debug_init_normal", C.c_int, [P, C.c_ulonglong, C.c_ulonglong, C.c_float])
 

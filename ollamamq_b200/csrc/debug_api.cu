@@ -347,6 +347,14 @@ int mq_debug_sample(const float* logits, int rows, int V, int ldl, int* out_toke
   return check_cuda("mq_debug_sample");
 }
 
+int mq_debug_sample_logprobs(const float* logits, int rows, int V, int ldl, int* out_tokens, const float* temperature,
+                             const int* top_k, const float* top_p, const unsigned long long* seed, const int* counter,
+                             const int* top_logprobs, void* lp_out) {
+  SampleCtl ctl{temperature, top_k, top_p, seed, counter, top_logprobs, (LogprobRec*)lp_out};
+  launch_sample(LaunchCfg{0, false}, logits, rows, V, ldl, out_tokens, nullptr, nullptr, nullptr, nullptr, ctl);
+  return check_cuda("mq_debug_sample_logprobs");
+}
+
 int mq_debug_argmax(const float* logits, int rows, int V, int ldl, int* out_tokens, const int* dst_slot,
                     int* cur_token, int* pos_inc, const int* active) {
   launch_argmax(LaunchCfg{0, false}, logits, rows, V, ldl, out_tokens, dst_slot, cur_token, pos_inc, active);

@@ -504,6 +504,8 @@ int mq_dispatcher_submit(mq_dispatcher* d, const char* user, const char* ip, con
       if (pb.has_top_k) t->rq.top_k = (int32_t)(pb.top_k < (1 << 30) ? pb.top_k : (1 << 30));
       if (pb.has_top_p) t->rq.top_p = (float)pb.top_p;
       if (pb.has_seed) t->rq.seed = pb.seed;
+      if (pb.has_logprobs) t->rq.logprobs = pb.logprobs ? 1 : 0;
+      if (pb.has_top_logprobs) t->rq.top_logprobs = (int16_t)pb.top_logprobs;
     }
   }
   {

@@ -155,6 +155,8 @@ static int worker_alloc(mq_worker* w) {
   CUDA_TRY(cudaMemsetAsync(w->d_topp, 0, MBp * 4, w->stream));
   CUDA_TRY(cudaMemsetAsync(w->d_topk, 0, MBp * 4, w->stream));
   CUDA_TRY(cudaMemsetAsync(w->d_seed, 0, MBp * 8, w->stream));
+  if ((rc = dalloc(&w->d_lp_top, MBp)) || (rc = dalloc(&w->d_lp_ring, (size_t)kRing * MBp))) return rc;
+  CUDA_TRY(cudaMemsetAsync(w->d_lp_top, 0xFF, MBp * 4, w->stream));  // -1: off
   if ((rc = dalloc(&w->d_identity, MBp))) return rc;
   if ((rc = dalloc(&w->d_block_table, (size_t)MBp * w->max_pages))) return rc;
   if ((rc = dalloc(&w->d_out_ring, (size_t)kRing * MBp))) return rc;
@@ -171,11 +173,14 @@ static int worker_alloc(mq_worker* w) {
   CUDA_TRY(cudaMallocHost((void**)&w->h_topk, MBp * 4));
   CUDA_TRY(cudaMallocHost((void**)&w->h_seed, MBp * 8));
   memset(w->h_temp, 0, MBp * 4); memset(w->h_topp, 0, MBp * 4); memset(w->h_topk, 0, MBp * 4); memset(w->h_seed, 0, MBp * 8);
+  CUDA_TRY(cudaMallocHost((void**)&w->h_lp_top, MBp * 4));
+  memset(w->h_lp_top, 0xFF, MBp * 4);
+  CUDA_TRY(cudaMallocHost((void**)&w->h_lp_ring, (size_t)kRing * MBp * sizeof(LogprobRec)));
   CUDA_TRY(cudaMallocHost((void**)&w->h_block_table, (size_t)MBp * w->max_pages * 4));
   memset(w->h_pos, 0, MBp * 4);
   memset(w->h_active, 0, MBp * 4);
   memset(w->h_block_table, 0, (size_t)MBp * w->max_pages * 4);
-  w->stage_ints = (size_t)3 * MT + 4 * (size_t)(MT + MB) + 10 * (size_t)MBp + (size_t)MBp * w->max_pages + 64;
+  w->stage_ints = (size_t)3 * MT + 4 * (size_t)(MT + MB) + 11 * (size_t)MBp + (size_t)MBp * w->max_pages + 64;
   CUDA_TRY(cudaMallocHost((void**)&w->h_stage, w->stage_ints * 4 * kStageSlots));
   CUDA_TRY(cudaMallocHost((void**)&w->h_out_ring, (size_t)kRing * MBp * 4));
   w->stage_ev.resize(kStageSlots);
@@ -526,15 +531,19 @@ static void upload_slots(mq_worker* w) {
   int* s_pos = st;
   int* s_act = st + MBp;
   int* s_bt = st + 2 * MBp;
-  int* s_samp = s_bt + (size_t)MBp * w->max_pages;  // temperature | top_k | top_p | seed (2 ints each)
+  // temperature | top_k | top_p | seed (2 ints each) | top_logprobs
+  int* s_samp = s_bt + (size_t)MBp * w->max_pages;
+  int* s_lp = s_samp + 5 * MBp + (MBp & 1);
   memcpy(s_samp, w->h_temp, MBp * 4);
   memcpy(s_samp + MBp, w->h_topk, MBp * 4);
   memcpy(s_samp + 2 * MBp, w->h_topp, MBp * 4);
   memcpy(s_samp + 3 * MBp + (MBp & 1), w->h_seed, MBp * 8);
+  memcpy(s_lp, w->h_lp_top, MBp * 4);
   cudaMemcpyAsync(w->d_temp, s_samp, MBp * 4, cudaMemcpyHostToDevice, w->stream);
   cudaMemcpyAsync(w->d_topk, s_samp + MBp, MBp * 4, cudaMemcpyHostToDevice, w->stream);
   cudaMemcpyAsync(w->d_topp, s_samp + 2 * MBp, MBp * 4, cudaMemcpyHostToDevice, w->stream);
   cudaMemcpyAsync(w->d_seed, s_samp + 3 * MBp + (MBp & 1), MBp * 8, cudaMemcpyHostToDevice, w->stream);
+  cudaMemcpyAsync(w->d_lp_top, s_lp, MBp * 4, cudaMemcpyHostToDevice, w->stream);
   memcpy(s_pos, w->h_pos, MBp * 4);
   memcpy(s_act, w->h_active, MBp * 4);
   memcpy(s_bt, w->h_block_table, (size_t)MBp * w->max_pages * 4);
@@ -560,6 +569,7 @@ static void free_slot(mq_worker* w, mq_req* r) {
   w->slot_req[s] = nullptr;
   w->h_active[s] = 0;
   w->h_pos[s] = 0;
+  w->h_lp_top[s] = -1;
   for (int i = 0; i < w->max_pages; ++i) w->h_block_table[(size_t)s * w->max_pages + i] = 0;  // scratch page
   w->slots_dirty = true;
   r->slot = -1;
@@ -580,14 +590,15 @@ static void finish_req(mq_worker* w, mq_req* r, int rc, const char* msg) {
   if (rc == 0) {
     send_status(r);
     std::string tail = frame_final(r->rq.endpoint, r->rq.stream, w->cfg.model_name, r->agg, (int)r->prompt.size(),
-                                   r->n_emitted, r->stopped);
+                                   r->n_emitted, r->stopped, r->top_logprobs >= 0 ? &r->agg_lp : nullptr);
     if (!tail.empty() && r->cb.on_chunk) r->cb.on_chunk(r->user, (const uint8_t*)tail.data(), tail.size());
   }
   if (r->cb.on_done) r->cb.on_done(r->user, rc, msg ? msg : "");
   req_unref(r);
 }
 
-static void emit_token(mq_worker* w, mq_req* r, int tok) {
+// rec: the token's log-probability record (read only when the request asked for one)
+static void emit_token(mq_worker* w, mq_req* r, int tok, const LogprobRec* rec) {
   if (r->finished) return;
   if (!r->rq.ignore_eos && w->cfg.eos_token_id > 0 && tok == w->cfg.eos_token_id) {
     // end of sequence: the EOS token itself is not relayed; steps already in flight for this slot are discarded
@@ -599,7 +610,22 @@ static void emit_token(mq_worker* w, mq_req* r, int tok) {
   if (r->n_emitted == 0) r->t_first = Clock::now();
   r->n_emitted++;
   send_status(r);
-  if (r->rq.stream) {
+  if (r->top_logprobs >= 0) {
+    TokenLogprobs e;
+    e.id = tok;
+    e.logprob = rec->logprob;
+    for (int j = 0; j < r->top_logprobs; ++j) e.top.push_back({rec->id[j], rec->lp[j]});
+    std::string s;
+    if (r->rq.endpoint == MQ_EP_RAW_TOKENS) append_raw_record(r->rq.stream ? &s : &r->agg, e);
+    else if (r->rq.stream) s = frame_token(r->rq.endpoint, w->cfg.model_name, tok, &e, r->text_len);
+    else r->agg += token_text(tok);
+    r->text_len += token_text(tok).size();
+    if (r->rq.stream) {
+      if (r->cb.on_chunk && r->cb.on_chunk(r->user, (const uint8_t*)s.data(), s.size()) != 0) r->cancel.store(true);
+    } else if (r->rq.endpoint != MQ_EP_RAW_TOKENS) {
+      r->agg_lp.push_back(std::move(e));
+    }
+  } else if (r->rq.stream) {
     uint8_t raw[4];
     std::string s;
     const uint8_t* data;
@@ -688,10 +714,16 @@ static int launch_prefill(mq_worker* w, std::vector<PrefillItem>& items) {
     const LaunchCfg lc{w->stream, c.use_pdl != 0};
     // first generated token of each finished prompt: RNG position 0 (decode steps use the token position >= 1)
     launch_sample(lc, w->logits, n_last, c.vocab, c.vocab, w->d_out_ring + (size_t)ring * MBp, w->d_dst_slot,
-                  w->d_cur_token, nullptr, nullptr, SampleCtl{w->d_temp, w->d_topk, w->d_topp, w->d_seed, nullptr});
+                  w->d_cur_token, nullptr, nullptr,
+                  SampleCtl{w->d_temp, w->d_topk, w->d_topp, w->d_seed, nullptr, w->d_lp_top, w->d_lp_ring + (size_t)ring * MBp});
     ++nl;
     cudaMemcpyAsync(w->h_out_ring + (size_t)ring * MBp, w->d_out_ring + (size_t)ring * MBp, n_last * 4,
                     cudaMemcpyDeviceToHost, w->stream);
+    bool want_lp = false;
+    for (auto& it : items) want_lp |= it.completes && it.r->top_logprobs >= 0;
+    if (want_lp)
+      cudaMemcpyAsync(w->h_lp_ring + (size_t)ring * MBp, w->d_lp_ring + (size_t)ring * MBp, n_last * sizeof(LogprobRec),
+                      cudaMemcpyDeviceToHost, w->stream);
   }
   f.ev = ev_get(w);
   cudaEventRecord(f.ev, w->stream);
@@ -741,7 +773,8 @@ static int decode_body(mq_worker* w, int Bcap, int n_splits, int attn_stages, in
   // NOTE: the ring slot is baked into a captured graph, so graphs write to a fixed staging row (ring 0 of the
   // graph area) and the copy-out below moves it into the real ring slot.
   launch_sample(lc, w->logits, Bcap, c.vocab, c.vocab, w->d_out_ring + (size_t)ring * MBp, nullptr, w->d_cur_token,
-                w->d_pos, w->d_active, SampleCtl{w->d_temp, w->d_topk, w->d_topp, w->d_seed, w->d_pos});
+                w->d_pos, w->d_active,
+                SampleCtl{w->d_temp, w->d_topk, w->d_topp, w->d_seed, w->d_pos, w->d_lp_top, w->d_lp_ring + (size_t)ring * MBp});
   *nl += 1;
   return MQ_OK;
 }
@@ -750,9 +783,11 @@ static int launch_decode(mq_worker* w) {
   const int MBp = round_up(w->MB, 16);
   int hi = -1, max_ctx = 1, n_active = 0;
   double kv_tokens = 0;
+  bool want_lp = false;  // some emitted slot asked for logprobs: copy the record row out beside the tokens
   for (int s = 0; s < w->MB; ++s)
     if (w->h_active[s]) {
       hi = s;
+      want_lp |= w->slot_req[s]->top_logprobs >= 0;
       ++n_active;
       max_ctx = std::max(max_ctx, w->h_pos[s] + 1);
       kv_tokens += w->h_pos[s] + 1;
@@ -827,12 +862,18 @@ static int launch_decode(mq_worker* w) {
     // graph wrote to the fixed row kRing-1; move it to this step's ring slot on the host side copy
     cudaMemcpyAsync(w->h_out_ring + (size_t)ring * MBp, w->d_out_ring + (size_t)(kRing - 1) * MBp, Bcap * 4,
                     cudaMemcpyDeviceToHost, w->stream);
+    if (want_lp)
+      cudaMemcpyAsync(w->h_lp_ring + (size_t)ring * MBp, w->d_lp_ring + (size_t)(kRing - 1) * MBp,
+                      Bcap * sizeof(LogprobRec), cudaMemcpyDeviceToHost, w->stream);
     nl = get_plans(w, Bcap, true)->chain ? (uint64_t)(1 + w->cfg.n_layers * 6 + 2) : (uint64_t)(1 + w->cfg.n_layers * 8 + 3);
   } else {
     int rc = decode_body(w, Bcap, n_splits, attn_stages, ring, &nl);
     if (rc) return rc;
     cudaMemcpyAsync(w->h_out_ring + (size_t)ring * MBp, w->d_out_ring + (size_t)ring * MBp, Bcap * 4,
                     cudaMemcpyDeviceToHost, w->stream);
+    if (want_lp)
+      cudaMemcpyAsync(w->h_lp_ring + (size_t)ring * MBp, w->d_lp_ring + (size_t)ring * MBp, Bcap * sizeof(LogprobRec),
+                      cudaMemcpyDeviceToHost, w->stream);
   }
   f.ev = ev_get(w);
   cudaEventRecord(f.ev, w->stream);
@@ -881,11 +922,12 @@ static void retire_flight(mq_worker* w, mq_worker::Flight& f) {
   }
   w->ev_pool.push_back(f.ev);
   const int* row = w->h_out_ring + (size_t)f.ring * MBp;
+  const LogprobRec* lp_row = w->h_lp_ring + (size_t)f.ring * MBp;
   for (auto& em : f.emits) {
     mq_req* r = em.first;
     if (r->finished) continue;
     if (r->cancel.load()) continue;  // handled by the cancel sweep
-    emit_token(w, r, row[em.second]);
+    emit_token(w, r, row[em.second], lp_row + em.second);
   }
   for (auto& em : f.emits) req_unref(em.first);
 }
@@ -939,6 +981,7 @@ static bool admit(mq_worker* w, mq_req* r) {
   w->h_pos[slot] = 0;
   w->h_active[slot] = 0;
   w->h_temp[slot] = r->temperature; w->h_topk[slot] = r->top_k; w->h_topp[slot] = r->top_p; w->h_seed[slot] = r->seed;
+  w->h_lp_top[slot] = r->top_logprobs;
   w->slots_dirty = true;
   return true;
 }
@@ -1236,9 +1279,9 @@ void mq_worker_close(mq_worker* w) {
   void* bufs[] = {w->k_cache, w->v_cache, w->h, w->x, w->q, w->attn, w->act, w->x_last, w->qkv_part, w->proj_part,
                   w->logits, w->part_o, w->part_ml, w->inv_freq, w->d_tok, w->d_pos_tok, w->d_slot_tok, w->d_last_idx,
                   w->d_dst_slot, w->d_tiles, w->d_cur_token, w->d_pos, w->d_active, w->d_block_table, w->d_identity,
-                  w->d_out_ring, w->d_split_counter, w->ssq_e, w->ssq_o, w->ssq_d};
+                  w->d_out_ring, w->d_split_counter, w->ssq_e, w->ssq_o, w->ssq_d, w->d_lp_top, w->d_lp_ring};
   for (void* b : bufs) if (b) cudaFree(b);
-  void* pinned[] = {w->h_pos, w->h_active, w->h_block_table, w->h_stage, w->h_out_ring};
+  void* pinned[] = {w->h_pos, w->h_active, w->h_block_table, w->h_stage, w->h_out_ring, w->h_lp_top, w->h_lp_ring};
   for (void* b : pinned) if (b) cudaFreeHost(b);
   for (auto e : w->stage_ev) cudaEventDestroy(e);
   for (auto e : w->ev_pool) cudaEventDestroy(e);
@@ -1376,6 +1419,8 @@ int mq_submit(mq_worker* w, const mq_request* rq, const mq_callbacks* cb, void* 
   r->top_k = pb.has_top_k ? (int)std::min<long long>(pb.top_k, 1 << 30) : rq->top_k;
   r->top_p = pb.has_top_p ? (float)pb.top_p : rq->top_p;
   r->seed = pb.has_seed ? pb.seed : rq->seed;
+  if (pb.has_logprobs ? pb.logprobs : rq->logprobs != 0)
+    r->top_logprobs = pb.has_top_logprobs ? pb.top_logprobs : std::max(0, std::min<int>(rq->top_logprobs, MQ_TOP_LOGPROBS_MAX));
   if (!(r->temperature == r->temperature)) r->temperature = 0.f;  // NaN from a C-ABI caller: greedy
   if (!(r->top_p == r->top_p)) r->top_p = 0.f;
   if (((long long)r->prompt.size() + r->max_new + kPageSize - 1) / kPageSize > w->n_pages - 1) {

@@ -3,6 +3,7 @@
 // This is what stands where the reference has `reqwest -> remote Ollama` (dispatcher.rs:287-312).
 #pragma once
 #include "../../include/ollamamq_b200.h"
+#include "framing.hpp"
 #include "gemm_host.cuh"
 #include "kernels.cuh"
 #include <atomic>
@@ -63,6 +64,9 @@ struct mq_req {
   float temperature = 0.f, top_p = 0.f;  // sampling controls (0 = greedy / off)
   int top_k = 0;
   unsigned long long seed = 0;
+  int top_logprobs = -1;  // -1: no logprobs; 0..MQ_TOP_LOGPROBS_MAX: a record per relayed token with that many alternatives
+  size_t text_len = 0;    // characters relayed so far (/v1/completions text_offset)
+  std::vector<mq::TokenLogprobs> agg_lp;  // stream=0 with logprobs: every relayed token's entry
   std::atomic<bool> cancel{false};
   bool status_sent = false;
   bool finished = false;
@@ -107,7 +111,9 @@ struct mq_worker {
   float *d_temp = nullptr, *d_topp = nullptr, *h_temp = nullptr, *h_topp = nullptr;
   int *d_topk = nullptr, *h_topk = nullptr;
   unsigned long long *d_seed = nullptr, *h_seed = nullptr;
+  int *d_lp_top = nullptr, *h_lp_top = nullptr;  // top_logprobs per slot, -1 = off (read by the sampler, graphs included)
   int* d_out_ring = nullptr;  // [kRing][MB]
+  mq::LogprobRec* d_lp_ring = nullptr;  // [kRing][MB] records beside d_out_ring, copied out only when a slot asked
   int* d_split_counter = nullptr;  // [MB][n_kv] arrival counters of the split-KV decode attention
   // decode chain: per-weight-tile partial sums of h^2 (RMSNorm fold, gemm.cuh RstdIn), [tiles][round_up(MB, 16)]
   float *ssq_e = nullptr, *ssq_o = nullptr, *ssq_d = nullptr;
@@ -123,6 +129,7 @@ struct mq_worker {
   int *h_pos = nullptr, *h_active = nullptr, *h_block_table = nullptr;
   int* h_stage = nullptr;     // ring of staging areas for metadata uploads
   int* h_out_ring = nullptr;  // [kRing][MB]
+  mq::LogprobRec* h_lp_ring = nullptr;  // [kRing][MB]
   size_t stage_ints = 0;
   int stage_next = 0;
   std::vector<cudaEvent_t> stage_ev;
@@ -156,7 +163,7 @@ struct mq_worker {
     bool decode = false;
     int ring = 0;
     double bytes = 0;
-    std::vector<std::pair<mq_req*, int>> emits;  // (request, index into h_out_ring row)
+    std::vector<std::pair<mq_req*, int>> emits;  // (request, index into h_out_ring row and h_lp_ring row)
   };
   std::deque<Flight> flights;
   std::vector<cudaEvent_t> ev_pool;

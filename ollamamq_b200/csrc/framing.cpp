@@ -231,11 +231,33 @@ bool parse_sampling(J& j, const std::string& k, ParsedBody* out, bool* used) {
 }  // namespace
 
 bool parse_body(const std::string& body, int endpoint, ParsedBody* out) {
-  (void)endpoint;
   J j{body.data(), body.data() + body.size()};
+  const bool legacy_lp = endpoint == MQ_EP_V1_COMPLETIONS;  // "logprobs": N | null instead of true | false
+  int legacy_n = -1;
   const bool ok = j.object([&](const std::string& k) {
     bool used = false;
     if (k == "model") return j.at('"') ? j.str(&out->model) : j.skip();
+    if (k == "logprobs") {
+      j.ws();
+      if (legacy_lp) {
+        if (j.lit("null")) { out->has_logprobs = true; out->logprobs = false; legacy_n = -1; return true; }
+        double v;
+        bool got;
+        if (!j.number_or_skip(&v, &got)) return false;
+        if (got) { out->has_logprobs = out->logprobs = true; legacy_n = (int)clamp_num(v, 0.0, MQ_TOP_LOGPROBS_MAX); }
+        return true;
+      }
+      if (j.lit("true")) { out->has_logprobs = out->logprobs = true; return true; }
+      if (j.lit("false")) { out->has_logprobs = true; out->logprobs = false; return true; }
+      return j.skip();
+    }
+    if (k == "top_logprobs") {
+      double v;
+      bool got;
+      if (!j.number_or_skip(&v, &got)) return false;
+      if (got) { out->has_top_logprobs = true; out->top_logprobs = (int)clamp_num(v, 0.0, MQ_TOP_LOGPROBS_MAX); }
+      return true;
+    }
     if (k == "prompt") {
       if (j.at('[')) return j.int_array(&out->tokens);
       if (j.at('"')) return j.str(&out->text);
@@ -264,6 +286,7 @@ bool parse_body(const std::string& body, int endpoint, ParsedBody* out) {
     return j.skip();
   });
   if (!ok) return false;
+  if (legacy_n >= 0) { out->has_top_logprobs = true; out->top_logprobs = legacy_n; }
   j.ws();
   return j.p == j.e;  // nothing but whitespace after the object
 }
@@ -315,20 +338,90 @@ static std::string model_field(const char* model) {
   return json_escape(m);
 }
 
-std::string frame_token(int endpoint, const char* model, int tok) {
+// ---- token log-probabilities: Ollama's api.Logprob list on /api/*, OpenAI's choices[0].logprobs on /v1/*
+static char* put_float(char* w, float f);
+static void put_num(std::string& o, float f) {
+  char b[32];
+  o.append(b, (size_t)(put_float(b, f) - b));
+}
+static void lp_fields(std::string& o, int id, float lp) {  // "token":..,"logprob":..,"bytes":[..]
+  const std::string t = token_text(id);
+  o += "\"token\":\"" + json_escape(t) + "\",\"logprob\":";
+  put_num(o, lp);
+  o += ",\"bytes\":[";
+  for (size_t i = 0; i < t.size(); ++i) {
+    if (i) o += ',';
+    o += std::to_string((unsigned char)t[i]);
+  }
+  o += ']';
+}
+// the "logprobs" member of a reply carrying n entries; /v1/completions counts text_offset from off0
+static std::string lp_member(int endpoint, const TokenLogprobs* e, size_t n, size_t off0) {
+  if (endpoint == MQ_EP_V1_COMPLETIONS) {
+    std::string toks, lps, tops, offs;
+    size_t off = off0;
+    for (size_t i = 0; i < n; ++i) {
+      const char* sep = i ? "," : "";
+      const std::string t = token_text(e[i].id);
+      toks += sep; toks += "\"" + json_escape(t) + "\"";
+      lps += sep; put_num(lps, e[i].logprob);
+      tops += sep; tops += '{';
+      for (size_t j = 0; j < e[i].top.size(); ++j) {
+        if (j) tops += ',';
+        tops += "\"" + json_escape(token_text(e[i].top[j].first)) + "\":";
+        put_num(tops, e[i].top[j].second);
+      }
+      tops += '}';
+      offs += sep; offs += std::to_string(off);
+      off += t.size();
+    }
+    return "\"logprobs\":{\"tokens\":[" + toks + "],\"token_logprobs\":[" + lps + "],\"top_logprobs\":[" + tops +
+           "],\"text_offset\":[" + offs + "]}";
+  }
+  const bool chat = endpoint == MQ_EP_V1_CHAT;
+  std::string o = chat ? "\"logprobs\":{\"content\":[" : "\"logprobs\":[";
+  for (size_t i = 0; i < n; ++i) {
+    if (i) o += ',';
+    o += '{';
+    lp_fields(o, e[i].id, e[i].logprob);
+    o += ",\"top_logprobs\":[";
+    for (size_t j = 0; j < e[i].top.size(); ++j) {
+      if (j) o += ',';
+      o += '{';
+      lp_fields(o, e[i].top[j].first, e[i].top[j].second);
+      o += '}';
+    }
+    o += "]}";
+  }
+  return o + (chat ? "]}" : "]");
+}
+
+void append_raw_record(std::string* out, const TokenLogprobs& e) {
+  char b[8];
+  memcpy(b, &e.id, 4); memcpy(b + 4, &e.logprob, 4);
+  out->append(b, 8);
+  for (auto& t : e.top) {
+    memcpy(b, &t.first, 4); memcpy(b + 4, &t.second, 4);
+    out->append(b, 8);
+  }
+}
+
+std::string frame_token(int endpoint, const char* model, int tok, const TokenLogprobs* lp, size_t text_off) {
   const std::string m = model_field(model), txt = json_escape(token_text(tok));
+  const std::string lpm = lp ? "," + lp_member(endpoint, lp, 1, text_off) : std::string();
   switch (endpoint) {
     case MQ_EP_API_GENERATE:
-      return "{\"model\":\"" + m + "\",\"created_at\":\"" + now_iso() + "\",\"response\":\"" + txt + "\",\"done\":false}\n";
+      return "{\"model\":\"" + m + "\",\"created_at\":\"" + now_iso() + "\",\"response\":\"" + txt + "\",\"done\":false" + lpm + "}\n";
     case MQ_EP_API_CHAT:
       return "{\"model\":\"" + m + "\",\"created_at\":\"" + now_iso() + "\",\"message\":{\"role\":\"assistant\",\"content\":\"" + txt +
-             "\"},\"done\":false}\n";
+             "\"},\"done\":false" + lpm + "}\n";
     case MQ_EP_V1_CHAT:
       return "data: {\"id\":\"chatcmpl-mq\",\"object\":\"chat.completion.chunk\",\"created\":" + std::to_string((long)time(nullptr)) +
-             ",\"model\":\"" + m + "\",\"choices\":[{\"index\":0,\"delta\":{\"content\":\"" + txt + "\"},\"finish_reason\":null}]}\n\n";
+             ",\"model\":\"" + m + "\",\"choices\":[{\"index\":0,\"delta\":{\"content\":\"" + txt + "\"}" + lpm +
+             ",\"finish_reason\":null}]}\n\n";
     default:
       return "data: {\"id\":\"cmpl-mq\",\"object\":\"text_completion\",\"created\":" + std::to_string((long)time(nullptr)) +
-             ",\"model\":\"" + m + "\",\"choices\":[{\"text\":\"" + txt + "\",\"index\":0,\"finish_reason\":null}]}\n\n";
+             ",\"model\":\"" + m + "\",\"choices\":[{\"text\":\"" + txt + "\",\"index\":0" + lpm + ",\"finish_reason\":null}]}\n\n";
   }
 }
 
@@ -356,19 +449,20 @@ void other_route_response(const std::string& path, const char* model, int* statu
 }
 
 std::string frame_final(int endpoint, int stream, const char* model, const std::string& agg, int n_prompt, int n_gen,
-                        bool stopped) {
+                        bool stopped, const std::vector<TokenLogprobs>* lps) {
   const char* why = stopped ? "stop" : "length";  // EOS reached vs generation budget spent
   if (endpoint == MQ_EP_RAW_TOKENS) return stream ? std::string() : agg;
   const std::string m = model_field(model), txt = json_escape(agg);
+  const std::string lpm = lps && !stream ? "," + lp_member(endpoint, lps->data(), lps->size(), 0) : std::string();
   std::string o;
   char buf[256];  // integers and the fixed words only: cannot truncate
   if (endpoint == MQ_EP_API_GENERATE || endpoint == MQ_EP_API_CHAT) {
     o = "{\"model\":\"" + m + "\",\"created_at\":\"" + now_iso() + "\",";
     if (endpoint == MQ_EP_API_GENERATE) o += "\"response\":\"" + (stream ? std::string() : txt) + "\",";
     else o += "\"message\":{\"role\":\"assistant\",\"content\":\"" + (stream ? std::string() : txt) + "\"},";
-    snprintf(buf, sizeof(buf), "\"done\":true,\"done_reason\":\"%s\",\"prompt_eval_count\":%d,\"eval_count\":%d}\n",
+    snprintf(buf, sizeof(buf), "\"done\":true,\"done_reason\":\"%s\",\"prompt_eval_count\":%d,\"eval_count\":%d",
              why, n_prompt, n_gen);
-    return o + buf;
+    return o + buf + lpm + "}\n";
   }
   const bool chat = endpoint == MQ_EP_V1_CHAT;
   if (stream) {
@@ -383,10 +477,10 @@ std::string frame_final(int endpoint, int stream, const char* model, const std::
   if (chat)
     o = "{\"id\":\"chatcmpl-mq\",\"object\":\"chat.completion\",\"model\":\"" + m +
         "\",\"choices\":[{\"index\":0,\"message\":{\"role\":\"assistant\",\"content\":\"" + txt +
-        "\"},\"finish_reason\":\"" + std::string(why) + "\"}],";
+        "\"}" + lpm + ",\"finish_reason\":\"" + std::string(why) + "\"}],";
   else
     o = "{\"id\":\"cmpl-mq\",\"object\":\"text_completion\",\"model\":\"" + m + "\",\"choices\":[{\"text\":\"" + txt +
-        "\",\"index\":0,\"finish_reason\":\"" + std::string(why) + "\"}],";
+        "\",\"index\":0" + lpm + ",\"finish_reason\":\"" + std::string(why) + "\"}],";
   return o + buf;
 }
 
@@ -530,12 +624,15 @@ long long mq_debug_parse_body(int32_t endpoint, const uint8_t* body, size_t len,
   const std::vector<int32_t> t = !pb.tokens.empty() ? pb.tokens : byte_tokenize(pb.text, vocab > 0 ? vocab : 256);
   for (size_t i = 0; i < t.size(); ++i) toks += (i ? "," : "") + std::to_string(t[i]);
   toks += "]";
-  char b[512];
+  char b[640];
   snprintf(b, sizeof b, "{\"ok\":%s,\"has_stream\":%s,\"stream\":%s,\"num_predict\":%d,\"has_temperature\":%s,\"temperature\":%.9g,"
-           "\"has_top_k\":%s,\"top_k\":%lld,\"has_top_p\":%s,\"top_p\":%.9g,\"has_seed\":%s,\"seed\":%llu,\"n_text\":%zu,",
+           "\"has_top_k\":%s,\"top_k\":%lld,\"has_top_p\":%s,\"top_p\":%.9g,\"has_seed\":%s,\"seed\":%llu,\"n_text\":%zu,"
+           "\"has_logprobs\":%s,\"logprobs\":%s,\"has_top_logprobs\":%s,\"top_logprobs\":%d,",
            ok ? "true" : "false", pb.has_stream ? "true" : "false", pb.stream ? "true" : "false", pb.num_predict,
            pb.has_temperature ? "true" : "false", pb.temperature, pb.has_top_k ? "true" : "false", pb.top_k,
-           pb.has_top_p ? "true" : "false", pb.top_p, pb.has_seed ? "true" : "false", pb.seed, pb.text.size());
+           pb.has_top_p ? "true" : "false", pb.top_p, pb.has_seed ? "true" : "false", pb.seed, pb.text.size(),
+           pb.has_logprobs ? "true" : "false", pb.logprobs ? "true" : "false", pb.has_top_logprobs ? "true" : "false",
+           pb.top_logprobs);
   return emit_json(std::string(b) + "\"model\":\"" + json_escape(pb.model) + "\",\"tokens\":" + toks + "}", out, cap);
 }
 long long mq_debug_parse_embed(const uint8_t* body, size_t len, int32_t vocab, int32_t max_len, char* out, size_t cap) {
@@ -561,6 +658,46 @@ long long mq_debug_frame_embeddings(const char* path, const char* model, const f
 long long mq_debug_frame_final(int32_t endpoint, int32_t stream, const char* model, const char* agg, int32_t n_prompt,
                                int32_t n_gen, int32_t stopped, char* out, size_t cap) {
   return emit_json(mq::frame_final(endpoint, stream, model ? model : "", agg ? agg : "", n_prompt, n_gen, stopped != 0), out, cap);
+}
+long long mq_debug_frame_logprobs(int32_t endpoint, int32_t stream, const char* model, const int32_t* ids,
+                                  const float* records, int32_t n, int32_t top_logprobs, int32_t n_prompt, char* out,
+                                  size_t cap) {
+  using namespace mq;
+  const char* mdl = model ? model : "";
+  const bool on = top_logprobs >= 0;
+  std::vector<TokenLogprobs> lps;
+  std::string agg, o;
+  size_t text_len = 0;
+  for (int i = 0; i < n; ++i) {
+    TokenLogprobs e;
+    e.id = ids[i];
+    if (on) {
+      const float* r = records + (size_t)i * (1 + 2 * top_logprobs);
+      e.logprob = r[0];
+      for (int j = 0; j < top_logprobs; ++j) {
+        int id;
+        memcpy(&id, r + 1 + 2 * j, 4);
+        e.top.push_back({id, r[2 + 2 * j]});
+      }
+    }
+    if (stream) {
+      if (endpoint == MQ_EP_RAW_TOKENS) {
+        if (on) append_raw_record(&o, e);
+        else o.append((const char*)&e.id, 4);
+      } else {
+        o += frame_token(endpoint, mdl, e.id, on ? &e : nullptr, text_len);
+      }
+    } else if (endpoint == MQ_EP_RAW_TOKENS) {
+      if (on) append_raw_record(&agg, e);
+      else agg.append((const char*)&e.id, 4);
+    } else {
+      agg += token_text(e.id);
+    }
+    text_len += token_text(e.id).size();
+    lps.push_back(e);
+  }
+  o += frame_final(endpoint, stream, mdl, agg, n_prompt, n, false, on ? &lps : nullptr);
+  return emit_json(o, out, cap);  // (raw tokens: binary, the returned length minus the terminator)
 }
 }  // extern "C"
 

@@ -5,6 +5,7 @@
 #pragma once
 #include <cstdint>
 #include <string>
+#include <utility>
 #include <vector>
 
 namespace mq {
@@ -21,17 +22,35 @@ struct ParsedBody {
   double temperature = 0, top_p = 0;
   long long top_k = 0;
   unsigned long long seed = 0;
+  // token log-probabilities, top level only: "logprobs": true / false (/api/*, /v1/chat/completions) or N / null
+  // (/v1/completions, where N also sets top_logprobs); "top_logprobs": N.  N is clamped to 0..MQ_TOP_LOGPROBS_MAX.
+  bool has_logprobs = false, logprobs = false;
+  bool has_top_logprobs = false;
+  int top_logprobs = 0;
+};
+
+// One relayed token's log-probability entry: its own, and the top alternatives (logit descending, id ascending).
+struct TokenLogprobs {
+  int id = 0;
+  float logprob = 0.f;
+  std::vector<std::pair<int, float>> top;
 };
 
 bool parse_body(const std::string& body, int endpoint, ParsedBody* out);
 std::vector<int32_t> byte_tokenize(const std::string& text, int vocab);
 std::string token_text(int tok);
 const char* content_type_for(int endpoint, int stream);
-std::string frame_token(int endpoint, const char* model, int tok);
+// lp: the token's logprobs entry (nullptr = off: the frame is exactly the one without); text_off = characters of the
+// reply before this token (/v1/completions "text_offset")
+std::string frame_token(int endpoint, const char* model, int tok, const TokenLogprobs* lp = nullptr, size_t text_off = 0);
+// raw-token record (MQ_EP_RAW_TOKENS with logprobs): int32 id, float32 logprob, N x (int32 id, float32 logprob)
+void append_raw_record(std::string* out, const TokenLogprobs& e);
 // MQ_EP_OTHER: what the backend answers on the non-generation routes (main.rs:92-112) without touching the GPU
 void other_route_response(const std::string& path, const char* model, int* status, std::string* ctype, std::string* body);
+// stopped: done_reason / finish_reason "stop" (EOS) instead of "length".  lps: every token's entry, carried by the
+// stream = 0 reply (nullptr = off: the reply is exactly the one without)
 std::string frame_final(int endpoint, int stream, const char* model, const std::string& agg, int n_prompt, int n_gen,
-                        bool stopped = false);  // stopped: done_reason / finish_reason "stop" (EOS) instead of "length"
+                        bool stopped = false, const std::vector<TokenLogprobs>* lps = nullptr);
 
 // ---- embeddings (/api/embed, /api/embeddings, /v1/embeddings)
 struct ParsedEmbed {

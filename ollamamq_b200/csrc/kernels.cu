@@ -14,6 +14,7 @@
 //   attn_combine     merge the split-KV partials
 //   argmax           greedy sampler + device-side advance of (cur_token, pos) so decode steps chain on the GPU
 #include "kernels.cuh"
+#include <cfloat>
 #include <type_traits>
 #include <cstdlib>
 #include <algorithm>
@@ -1074,6 +1075,118 @@ __device__ void bitonic_desc(float* val, int* idx, int n /* power of two */) {
     }
 }
 
+// Steps a - c: elements >= the k-th largest of the 1024 thread maxima (0 < k <= 1024) are compacted into cval / cidx
+// and, when they fit (return value <= kSampleCand), sorted value descending / id ascending; a larger return value is
+// the count of a pool that overflowed.  want_z: *z_part = this thread's share of sum exp((l - mx) * inv_t) over the row.
+// Shared by the top-k path and the log-probability record.
+__device__ int gather_candidates(const float* __restrict__ lp, int V, float thread_max, int k, float* cval, int* cidx,
+                                 int* n_cand, bool want_z, float mx, float inv_t, float* z_part) {
+  cval[threadIdx.x] = thread_max;
+  cidx[threadIdx.x] = threadIdx.x;
+  if (threadIdx.x == 0) *n_cand = 0;
+  __syncthreads();
+  bitonic_desc(cval, cidx, 1024);
+  const float t0 = cval[k - 1];
+  __syncthreads();
+  float z = 0.f;  // fixed order per thread (the caller sums the threads in a fixed tree)
+  for (int i = threadIdx.x; i < V; i += blockDim.x) {
+    const float l = lp[i];
+    if (want_z) z += __expf((l - mx) * inv_t);
+    if (l >= t0) {
+      const int at = atomicAdd(n_cand, 1);
+      if (at < kSampleCand) { cval[at] = l; cidx[at] = i; }
+    }
+  }
+  *z_part = z;
+  __syncthreads();
+  const int nc = *n_cand;
+  if (nc <= kSampleCand) {
+    int n2 = 2;
+    while (n2 < nc) n2 <<= 1;
+    for (int i = nc + threadIdx.x; i < n2; i += blockDim.x) { cval[i] = -INFINITY; cidx[i] = 0x7fffffff; }
+    __syncthreads();
+    bitonic_desc(cval, cidx, n2);
+  }
+  return nc;
+}
+
+// The log-probability record of a row (see LogprobRec), before the draw while the pool is free: lse, then the n
+// (<= min(kTopLogprobsMax, V)) most probable tokens into rec->id / rec->lp.  Returns lse to every thread; the drawn
+// token's own entry is written beside the token.
+__device__ float logprob_record(const float* __restrict__ lp, int V, int n, LogprobRec* rec, float* cval, int* cidx,
+                                unsigned long long* hist, uint32_t* bcast, int* n_cand) {
+  __shared__ float wm[32], ws[32];
+  __shared__ int wc[32];
+  // per-thread online (max, sum exp(l - max)) over the thread's strided share, in a fixed order
+  float m = -FLT_MAX, s = 0.f;
+  for (int i = threadIdx.x; i < V; i += blockDim.x) {
+    const float l = lp[i];
+    if (l > m) { s = s * __expf(m - l) + 1.f; m = l; }
+    else s += __expf(l - m);
+  }
+  const float thread_max = m;
+  // fixed tree: xor butterfly inside the warp (both lanes of a pair compute the same bits), then the warps in order
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    const float om = __shfl_xor_sync(0xffffffffu, m, o), os = __shfl_xor_sync(0xffffffffu, s, o);
+    const float mm = fmaxf(m, om);
+    s = s * __expf(m - mm) + os * __expf(om - mm);
+    m = mm;
+  }
+  if ((threadIdx.x & 31) == 0) { wm[threadIdx.x >> 5] = m; ws[threadIdx.x >> 5] = s; }
+  __syncthreads();
+  m = wm[0];
+  s = ws[0];
+  for (int w = 1; w < (int)(blockDim.x >> 5); ++w) {
+    const float mm = fmaxf(m, wm[w]);
+    s = s * __expf(m - mm) + ws[w] * __expf(wm[w] - mm);
+    m = mm;
+  }
+  const float lse = m + logf(s);
+  if (n > 0) {
+    float unused;
+    const int nc = gather_candidates(lp, V, thread_max, n, cval, cidx, n_cand, false, 0.f, 1.f, &unused);
+    if (nc > kSampleCand) {
+      // a nearly flat row: the n-th largest key by the radix walk; every element above it (fewer than n) plus the
+      // lowest ids equal to it, collected in id order one block-wide chunk at a time
+      const uint32_t thr = radix_threshold<false>(lp, V, 0u, (unsigned long long)n, 0.f, 1.f, hist, bcast);
+      if (threadIdx.x == 0) *n_cand = 0;
+      __syncthreads();
+      for (int i = threadIdx.x; i < V; i += blockDim.x) {
+        const float l = lp[i];
+        if (f32_key(l) > thr) {
+          const int at = atomicAdd(n_cand, 1);
+          cval[at] = l; cidx[at] = i;
+        }
+      }
+      __syncthreads();
+      int have = *n_cand;
+      for (int base = 0; base < V && have < n; base += blockDim.x) {
+        const int i = base + threadIdx.x;
+        const bool eq = i < V && f32_key(lp[i]) == thr;
+        const unsigned bal = __ballot_sync(0xffffffffu, eq);
+        if ((threadIdx.x & 31) == 0) wc[threadIdx.x >> 5] = __popc(bal);
+        __syncthreads();
+        int before = 0, tot = 0;
+        for (int w = 0; w < (int)(blockDim.x >> 5); ++w) {
+          if (w < (int)(threadIdx.x >> 5)) before += wc[w];
+          tot += wc[w];
+        }
+        const int at = have + before + __popc(bal & ((1u << (threadIdx.x & 31)) - 1u));
+        if (eq && at < n) { cval[at] = lp[i]; cidx[at] = i; }
+        have += tot;
+        __syncthreads();
+      }
+      for (int i = n + threadIdx.x; i < 32; i += blockDim.x) { cval[i] = -INFINITY; cidx[i] = 0x7fffffff; }
+      __syncthreads();
+      bitonic_desc(cval, cidx, 32);
+    }
+    if ((int)threadIdx.x < n) { rec->id[threadIdx.x] = cidx[threadIdx.x]; rec->lp[threadIdx.x] = cval[threadIdx.x] - lse; }
+    __syncthreads();  // the draw reuses the pool
+  }
+  return lse;
+}
+
 __global__ void __launch_bounds__(1024) sample_kernel(const float* __restrict__ logits, int V, int ldl,
                                                       int* __restrict__ out_tokens, const int* __restrict__ dst_slot,
                                                       int* __restrict__ cur_token, int* __restrict__ pos_inc,
@@ -1093,6 +1206,10 @@ __global__ void __launch_bounds__(1024) sample_kernel(const float* __restrict__ 
   const int row = blockIdx.x;
   const int slot = dst_slot ? dst_slot[row] : row;
   const float* lp = logits + (size_t)row * ldl;
+  const int n_top = ctl.top_logprobs && ctl.lp_out ? ctl.top_logprobs[slot] : -1;
+  LogprobRec* rec = n_top >= 0 ? ctl.lp_out + row : nullptr;
+  float lse = 0.f;
+  if (rec) lse = logprob_record(lp, V, min(min(n_top, kTopLogprobsMax), V), rec, cval, cidx, hist, bcast, &n_cand);
   const float temp = ctl.temperature ? ctl.temperature[slot] : 0.f;
   const bool greedy = !(temp > 0.f);
   const float inv_t = greedy ? 1.f : 1.f / temp;
@@ -1127,35 +1244,15 @@ __global__ void __launch_bounds__(1024) sample_kernel(const float* __restrict__ 
     const int k_eff = (k > 0 && k <= 1024 && k < V) ? k : ((k <= 0 || k >= V) && p_on && V > 1024 ? 256 : 0);
     const bool p_only = k_eff > 0 && !(k > 0 && k < V);
     if (k_eff > 0 && blockDim.x == 1024) {
-      cval[threadIdx.x] = thread_max;
-      cidx[threadIdx.x] = threadIdx.x;
-      if (threadIdx.x == 0) n_cand = 0;
-      __syncthreads();
-      bitonic_desc(cval, cidx, 1024);
-      const float t0 = cval[k_eff - 1];
-      __syncthreads();
-      float zpart = 0.f;  // top-p alone: mass of the whole row (fixed order per thread, fixed tree below)
-      for (int i = threadIdx.x; i < V; i += blockDim.x) {
-        const float l = lp[i];
-        if (p_only) zpart += __expf((l - mx) * inv_t);
-        if (l >= t0) {
-          const int at = atomicAdd(&n_cand, 1);
-          if (at < kSampleCand) { cval[at] = l; cidx[at] = i; }
-        }
-      }
+      float zpart;  // top-p alone: mass of the whole row
+      const int nc = gather_candidates(lp, V, thread_max, k_eff, cval, cidx, &n_cand, p_only, mx, inv_t, &zpart);
       zpart = warp_sum(zpart);
       if ((threadIdx.x & 31) == 0) sb[threadIdx.x >> 5] = zpart;
       __syncthreads();
       float z_row = 0.f;
       for (int w = 0; w < (int)(blockDim.x >> 5); ++w) z_row += sb[w];
-      const int nc = n_cand;
       __syncthreads();
       if (nc <= kSampleCand) {
-        int n2 = 2;
-        while (n2 < nc) n2 <<= 1;
-        for (int i = nc + threadIdx.x; i < n2; i += blockDim.x) { cval[i] = -INFINITY; cidx[i] = 0x7fffffff; }
-        __syncthreads();
-        bitonic_desc(cval, cidx, n2);
         if (threadIdx.x == 0) {
           int nk = nc;
           if (!p_only) {
@@ -1237,6 +1334,7 @@ __global__ void __launch_bounds__(1024) sample_kernel(const float* __restrict__ 
           for (int w = 1; w < (int)(blockDim.x >> 5); ++w)
             if (sb[w] > best || (sb[w] == best && si[w] < bi)) { best = sb[w]; bi = si[w]; }
           out_tokens[row] = bi;
+          if (rec) rec->logprob = lp[bi] - lse;
           if (cur_token) cur_token[slot] = bi;
           if (pos_inc && (!active || active[slot])) pos_inc[slot] += 1;
         }
@@ -1301,6 +1399,7 @@ __global__ void __launch_bounds__(1024) sample_kernel(const float* __restrict__ 
       if (sb[w] > best || (sb[w] == best && si[w] < bi)) { best = sb[w]; bi = si[w]; }
     if (bi == 0x7fffffff) bi = 0;  // (cannot happen: the maximum is always kept)
     out_tokens[row] = bi;
+    if (rec) rec->logprob = lp[bi] - lse;
     if (cur_token) cur_token[slot] = bi;
     if (pos_inc && (!active || active[slot])) pos_inc[slot] += 1;
   }

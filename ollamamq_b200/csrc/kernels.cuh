@@ -117,14 +117,31 @@ void launch_enc_add_ln_warp(const LaunchCfg& lc, __nv_bfloat16* x, const __nv_bf
                             const __nv_bfloat16* g, const __nv_bfloat16* b, float* h32, int T, int H, float eps);
 void launch_enc_pool(const LaunchCfg& lc, const float* h, const int* first_tok, float* out, int n_seq, int H);
 
+// Log-probability record of one drawn token (MQ_TOP_LOGPROBS_MAX alternatives at most).  For the logits row l the token
+// was drawn from: logprob(i) = l[i] - lse(l), lse(l) = m + log sum_j exp(l[j] - m), m = max l - the log-softmax of the
+// raw logits (temperature 1, before top-k / top-p), whatever the request's sampling settings.  `logprob` is the drawn
+// token's; id[0..n) / lp[0..n) are the n most probable tokens, logit descending then id ascending (ties at the cut go
+// to the lower id), entries from n on are not written.  Fixed-order reductions: the same row gives the same bits.
+constexpr int kTopLogprobsMax = 20;
+struct LogprobRec {
+  float logprob;
+  int id[kTopLogprobsMax];
+  float lp[kTopLogprobsMax];
+};
+static_assert(sizeof(LogprobRec) == 4 + 8 * kTopLogprobsMax, "LogprobRec is the raw-token record layout");
+
 // Per-slot sampling controls (device arrays indexed by slot; a null array = the default): temperature <= 0 -> greedy;
 // top_k <= 0 or >= V -> off; top_p <= 0 or >= 1 -> off; counter = position of the token being drawn (RNG stream).
+// top_logprobs: -1 (or a null array) -> no record; 0..20 -> row r writes lp_out[r] with that many alternatives.  The
+// switch never changes the drawn token.
 struct SampleCtl {
   const float* temperature;
   const int* top_k;
   const float* top_p;
   const unsigned long long* seed;
   const int* counter;
+  const int* top_logprobs;
+  LogprobRec* lp_out;
 };
 // like launch_argmax, but rows whose slot has temperature > 0 are drawn from softmax(logits / T) restricted by
 // top-k / top-p (Gumbel-max with a counter-based generator: no state, reproducible per (seed, position))

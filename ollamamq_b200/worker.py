@@ -56,6 +56,7 @@ class Stream:
         self.t_submit = time.perf_counter()
         self.t_done = None
         self.handle = None
+        self.top_logprobs = -1   # >= 0: the request asked for logprobs (raw chunks are then records, see tokens())
 
         def _status(_u, code, ctype):
             self.status, self.content_type = code, (ctype or b"").decode()
@@ -85,10 +86,25 @@ class Stream:
     def body(self) -> bytes:
         return b"".join(self.chunks)
 
+    def _records(self):
+        import numpy as np
+        n = self.top_logprobs
+        rec = np.dtype([("id", "<i4"), ("logprob", "<f4"), ("top", [("id", "<i4"), ("logprob", "<f4")], (n,))])
+        return np.frombuffer(self.body, dtype=rec)
+
     def tokens(self) -> List[int]:
+        """Token ids of a raw-token reply (4-byte ids, or the ids of the logprob records when logprobs were asked)."""
         import struct
+        if self.top_logprobs >= 0:
+            return [int(t) for t in self._records()["id"]]
         b = self.body
         return list(struct.unpack("<%di" % (len(b) // 4), b))
+
+    def logprobs(self) -> List[tuple]:
+        """Raw-token reply of a request with logprobs: (logprob, [(id, logprob), ...top_logprobs]) per token."""
+        if self.top_logprobs < 0:
+            raise ValueError("the request did not ask for logprobs")
+        return [(float(r["logprob"]), [(int(t["id"]), float(t["logprob"])) for t in r["top"]]) for r in self._records()]
 
     @property
     def ttft(self) -> Optional[float]:
@@ -97,12 +113,14 @@ class Stream:
 
 def make_request(endpoint=EP_RAW_TOKENS, prompt_tokens: Optional[Sequence[int]] = None, body: Optional[bytes] = None,
                  max_new_tokens=16, stream=1, timeout_ms=0, path: Optional[str] = None, temperature=0.0, top_k=0,
-                 top_p=0.0, seed=0, ignore_eos=1):
+                 top_p=0.0, seed=0, ignore_eos=1, logprobs=False, top_logprobs=0):
     r = _lib.Request()
     if path is not None:
         r.path = path.encode()
     r.endpoint, r.stream, r.max_new_tokens, r.ignore_eos, r.timeout_ms = endpoint, stream, max_new_tokens, ignore_eos, timeout_ms
     r.temperature, r.top_k, r.top_p, r.seed = float(temperature), int(top_k), float(top_p), int(seed)
+    r.logprobs = 1 if logprobs else 0
+    r.top_logprobs = max(0, min(int(top_logprobs), _lib.MQ_TOP_LOGPROBS_MAX))
     keep = []
     if body is not None:
         buf = C.create_string_buffer(body, len(body))
@@ -170,22 +188,26 @@ class Worker:
         return out
 
     def submit(self, sink: Stream, **kw) -> Stream:
-        """kw: endpoint, prompt_tokens, body, max_new_tokens, stream (1/0/-1), timeout_ms."""
+        """kw: endpoint, prompt_tokens, body, max_new_tokens, stream (1/0/-1), timeout_ms, sampling, logprobs /
+        top_logprobs."""
         r, keep = make_request(**kw)
         h = C.c_void_p()
+        sink.top_logprobs = r.top_logprobs if r.logprobs else -1
         sink.t_submit = time.perf_counter()
         check(lib.mq_submit(self._h, C.byref(r), C.byref(sink.cb), None, C.byref(h)))
         sink.handle = h
         sink._worker = self
         return sink
 
-    def generate(self, prompt_tokens: Sequence[int], max_new_tokens: int, timeout=120) -> List[int]:
-        s = self.submit(Stream(), prompt_tokens=list(prompt_tokens), max_new_tokens=max_new_tokens)
+    def generate(self, prompt_tokens: Sequence[int], max_new_tokens: int, timeout=120, logprobs=False, top_logprobs=0):
+        """Token ids; with logprobs=True, (token ids, Stream.logprobs())."""
+        s = self.submit(Stream(), prompt_tokens=list(prompt_tokens), max_new_tokens=max_new_tokens, logprobs=logprobs,
+                        top_logprobs=top_logprobs)
         s.wait(timeout)
         lib.mq_req_release(s.handle)
         if s.rc != 0:
             raise MQError(s.rc, s.err)
-        return s.tokens()
+        return (s.tokens(), s.logprobs()) if logprobs else s.tokens()
 
     def stats(self) -> dict:
         st = _lib.WorkerStats()
@@ -305,6 +327,7 @@ class Dispatcher:
     def submit(self, user: Optional[str], sink: Optional[Stream] = None, ip: Optional[str] = None, **kw) -> Stream:
         sink = sink or Stream()
         r, keep = make_request(**kw)
+        sink.top_logprobs = r.top_logprobs if r.logprobs else -1
         tid = C.c_uint64()
         sink.t_submit = time.perf_counter()
         check(lib.mq_dispatcher_submit(self._h, None if user is None else user.encode(),
