@@ -498,14 +498,7 @@ int mq_dispatcher_submit(mq_dispatcher* d, const char* user, const char* ip, con
     } else {
       if (!pb.tokens.empty()) { t->tokens = pb.tokens; t->body.clear(); }
       else { t->body.assign(pb.text.begin(), pb.text.end()); t->rq.body_kind = MQ_BODY_TEXT; }
-      if (pb.has_stream && t->rq.stream < 0) t->rq.stream = pb.stream ? 1 : 0;
-      if (t->rq.max_new_tokens <= 0 && pb.num_predict > 0) t->rq.max_new_tokens = pb.num_predict;
-      if (pb.has_temperature) t->rq.temperature = (float)pb.temperature;
-      if (pb.has_top_k) t->rq.top_k = (int32_t)(pb.top_k < (1 << 30) ? pb.top_k : (1 << 30));
-      if (pb.has_top_p) t->rq.top_p = (float)pb.top_p;
-      if (pb.has_seed) t->rq.seed = pb.seed;
-      if (pb.has_logprobs) t->rq.logprobs = pb.logprobs ? 1 : 0;
-      if (pb.has_top_logprobs) t->rq.top_logprobs = (int16_t)pb.top_logprobs;
+      apply_body(pb, &t->rq);
     }
   }
   {

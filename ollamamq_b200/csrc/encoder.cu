@@ -54,6 +54,7 @@ struct mq_encoder {
   mq_encoder_cfg cfg{};
   int gpu = 0;
   cudaStream_t stream = nullptr;
+  Allocations allocs;  // every buffer below (weights included) is owned here
   std::map<std::string, DevTensor> tensors;
   __nv_bfloat16 *word = nullptr, *pos_emb = nullptr, *type_emb = nullptr, *emb_g = nullptr, *emb_b = nullptr;
   std::vector<EncLayer> layers;
@@ -88,18 +89,8 @@ struct mq_encoder {
 
 namespace {
 
-template <typename T>
-int enc_alloc(T** p, size_t n) {
-  void* q = nullptr;
-  if (cudaMalloc(&q, n * sizeof(T)) != cudaSuccess) {
-    set_last_error("cudaMalloc(%zu bytes) failed", n * sizeof(T));
-    return MQ_ERR_NOMEM;
-  }
-  *p = (T*)q;
-  return MQ_OK;
-}
 int enc_tensor(mq_encoder* e, const std::string& name, size_t n, __nv_bfloat16** out) {
-  int rc = enc_alloc(out, n);
+  int rc = e->allocs.dev(out, n);
   if (rc) return rc;
   e->tensors[name] = DevTensor{*out, n * 2};
   return MQ_OK;
@@ -136,9 +127,10 @@ int enc_setup(mq_encoder* e) {
   e->MT = (std::max(c.max_tokens_per_pass, c.max_seq) + 255) / 256 * 256;
   e->max_seqs = std::max(1, std::min(1024, e->MT / 8));
   const size_t MT = e->MT;
-  if ((rc = enc_alloc(&e->h, MT * H))) return rc;
-  if ((rc = enc_alloc(&e->x, MT * H))) return rc;
-  if ((rc = enc_alloc(&e->qkv, MT * 3 * H))) return rc;
+  Allocations& m = e->allocs;
+  if ((rc = m.dev(&e->h, MT * H))) return rc;
+  if ((rc = m.dev(&e->x, MT * H))) return rc;
+  if ((rc = m.dev(&e->qkv, MT * 3 * H))) return rc;
   // the tcgen05 attention loads whole 64-row boxes: rows past a pass's last token must hold finite values (they meet
   // probabilities of exactly 0)
   ENC_TRY(cudaMemset(e->qkv, 0, MT * 3 * H * sizeof(__nv_bfloat16)));
@@ -148,15 +140,15 @@ int enc_setup(mq_encoder* e) {
   if (e->attn_tc) enc_attn_tc_set_attrs();
   const char* rl_env = getenv("MQ_ENC_ROWLN");
   e->rowln = rowln_supported(H, H) && rowln_supported(H, I) && !(rl_env && rl_env[0] == '0');
-  if ((rc = enc_alloc(&e->attn, MT * H))) return rc;
-  if ((rc = enc_alloc(&e->sub, MT * H))) return rc;
-  if ((rc = enc_alloc(&e->act, MT * I))) return rc;
-  if ((rc = enc_alloc(&e->d_out, (size_t)e->max_seqs * H))) return rc;
+  if ((rc = m.dev(&e->attn, MT * H))) return rc;
+  if ((rc = m.dev(&e->sub, MT * H))) return rc;
+  if ((rc = m.dev(&e->act, MT * I))) return rc;
+  if ((rc = m.dev(&e->d_out, (size_t)e->max_seqs * H))) return rc;
   const size_t max_tiles = MT / kEncTileRows + e->max_seqs + 1;
   e->meta_ints = 2 * MT + 2 * (size_t)e->max_seqs + 4 * max_tiles;
-  if ((rc = enc_alloc(&e->d_meta, e->meta_ints))) return rc;
-  ENC_TRY(cudaMallocHost((void**)&e->h_meta, e->meta_ints * 4));
-  ENC_TRY(cudaMallocHost((void**)&e->h_out, (size_t)e->max_seqs * H * 4));
+  if ((rc = m.dev(&e->d_meta, e->meta_ints)) || (rc = m.host(&e->h_meta, e->meta_ints)) ||
+      (rc = m.host(&e->h_out, (size_t)e->max_seqs * H)))
+    return rc;
   return MQ_OK;
 }
 
@@ -409,11 +401,8 @@ void mq_encoder_close(mq_encoder* e) {
   e->reply_cv.notify_all();
   if (e->reply_thr.joinable()) e->reply_thr.join();
   cudaSetDevice(e->gpu);
-  for (auto& kv : e->tensors) cudaFree(kv.second.ptr);
-  void* bufs[] = {e->h, e->d_out, e->x, e->qkv, e->attn, e->sub, e->act, e->d_meta};
-  for (void* b : bufs) if (b) cudaFree(b);
-  if (e->h_meta) cudaFreeHost(e->h_meta);
-  if (e->h_out) cudaFreeHost(e->h_out);
+  if (e->stream) cudaStreamSynchronize(e->stream);
+  e->allocs.free_all();
   if (e->ev0) cudaEventDestroy(e->ev0);
   if (e->ev1) cudaEventDestroy(e->ev1);
   if (e->stream) cudaStreamDestroy(e->stream);

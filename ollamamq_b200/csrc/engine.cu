@@ -28,25 +28,46 @@ static int round_up(int a, int b) { return (a + b - 1) / b * b; }
 // ------------------------------------------------------------------------------------------------
 // allocation / weights
 // ------------------------------------------------------------------------------------------------
-template <typename T>
-static int dalloc(T** p, size_t n_elems) {
+int Allocations::alloc(void** p, size_t bytes, bool pinned_host) {
   void* q = nullptr;
-  cudaError_t e = cudaMalloc(&q, n_elems * sizeof(T));
+  const cudaError_t e = pinned_host ? cudaMallocHost(&q, bytes) : cudaMalloc(&q, bytes);
   if (e != cudaSuccess) {
-    set_last_error("cudaMalloc(%zu bytes): %s", n_elems * sizeof(T), cudaGetErrorString(e));
+    set_last_error("%s(%zu bytes): %s", pinned_host ? "cudaMallocHost" : "cudaMalloc", bytes, cudaGetErrorString(e));
     return MQ_ERR_NOMEM;
   }
-  *p = reinterpret_cast<T*>(q);
+  (pinned_host ? host_ptrs : dev_ptrs).push_back(q);
+  *p = q;
   return MQ_OK;
 }
 
+void Allocations::free_all() {
+  for (void* p : dev_ptrs) cudaFree(p);
+  for (void* p : host_ptrs) cudaFreeHost(p);
+  dev_ptrs.clear();
+  host_ptrs.clear();
+}
+
 static int add_tensor(mq_worker* w, const std::string& name, size_t n_elems, __nv_bfloat16** out) {
-  __nv_bfloat16* p = nullptr;
-  int rc = dalloc(&p, n_elems);
+  int rc = w->allocs.dev(out, n_elems);
   if (rc) return rc;
-  w->tensors[name] = DevTensor{p, n_elems * 2};
-  *out = p;
+  w->tensors[name] = DevTensor{*out, n_elems * 2};
   return MQ_OK;
+}
+
+// points views[0..] at consecutive sections of n entries each, starting at `at`; returns the end of the last section
+template <typename... T>
+static uint8_t* carve(uint8_t* at, size_t n, T**... views) {
+  ((*views = reinterpret_cast<T*>(at), at += n * sizeof(T)), ...);
+  return at;
+}
+
+// a slot's sampling entry in the slot table's host mirror
+static void set_slot_sampling(mq_worker* w, int s, const SamplingParams& p) {
+  w->h_temp[s] = p.temperature;
+  w->h_topk[s] = p.top_k;
+  w->h_topp[s] = p.top_p;
+  w->h_seed[s] = p.seed;
+  w->h_lp_top[s] = p.top_logprobs;
 }
 
 static int decode_splits(int m_tiles, int k_blocks) {
@@ -88,8 +109,9 @@ static int worker_alloc(mq_worker* w) {
   w->kv_bytes_per_tok = 2.0 * L * c.n_kv_heads * D * 2.0;
 
   w->cache_layer_stride = (size_t)w->n_pages * c.n_kv_heads * kPageSize * D;
-  if ((rc = dalloc(&w->k_cache, w->cache_layer_stride * L))) return rc;
-  if ((rc = dalloc(&w->v_cache, w->cache_layer_stride * L))) return rc;
+  Allocations& m = w->allocs;
+  if ((rc = m.dev(&w->k_cache, w->cache_layer_stride * L))) return rc;
+  if ((rc = m.dev(&w->v_cache, w->cache_layer_stride * L))) return rc;
   cudaMemsetAsync(w->k_cache, 0, w->cache_layer_stride * L * 2, w->stream);
   cudaMemsetAsync(w->v_cache, 0, w->cache_layer_stride * L * 2, w->stream);
 
@@ -101,27 +123,27 @@ static int worker_alloc(mq_worker* w) {
   const int s_o = decode_splits((H + 127) / 128, kbQ);
   const int s_d = decode_splits((H + 127) / 128, kbI);
   const int MBp = round_up(MB, 16);
-  if ((rc = dalloc(&w->h, (size_t)MT * H))) return rc;
-  if ((rc = dalloc(&w->x, (size_t)MT * H))) return rc;
-  if ((rc = dalloc(&w->q, (size_t)MT * qd))) return rc;
-  if ((rc = dalloc(&w->attn, (size_t)MT * qd))) return rc;
-  if ((rc = dalloc(&w->act, (size_t)MT * I))) return rc;
-  if ((rc = dalloc(&w->x_last, (size_t)MBp * H))) return rc;
+  if ((rc = m.dev(&w->h, (size_t)MT * H))) return rc;
+  if ((rc = m.dev(&w->x, (size_t)MT * H))) return rc;
+  if ((rc = m.dev(&w->q, (size_t)MT * qd))) return rc;
+  if ((rc = m.dev(&w->attn, (size_t)MT * qd))) return rc;
+  if ((rc = m.dev(&w->act, (size_t)MT * I))) return rc;
+  if ((rc = m.dev(&w->x_last, (size_t)MBp * H))) return rc;
   const size_t qkv_bytes = std::max((size_t)MT * w->qkv_dim * 2, (size_t)s_qkv * MBp * w->qkv_dim * 4);
   const size_t proj_bytes = std::max((size_t)MT * H * 2, (size_t)std::max(s_o, s_d) * MBp * H * 4);
   uint8_t* tmp;
-  if ((rc = dalloc(&tmp, qkv_bytes))) return rc;
+  if ((rc = m.dev(&tmp, qkv_bytes))) return rc;
   w->qkv_part = tmp;
-  if ((rc = dalloc(&tmp, proj_bytes))) return rc;
+  if ((rc = m.dev(&tmp, proj_bytes))) return rc;
   w->proj_part = tmp;
-  if ((rc = dalloc(&w->logits, (size_t)MBp * V))) return rc;
-  if ((rc = dalloc(&w->part_o, (size_t)kMaxDecodeSplits * MBp * c.n_q_heads * D))) return rc;
-  if ((rc = dalloc(&w->part_ml, (size_t)kMaxDecodeSplits * MBp * c.n_q_heads * 2))) return rc;
+  if ((rc = m.dev(&w->logits, (size_t)MBp * V))) return rc;
+  if ((rc = m.dev(&w->part_o, (size_t)kMaxDecodeSplits * MBp * c.n_q_heads * D))) return rc;
+  if ((rc = m.dev(&w->part_ml, (size_t)kMaxDecodeSplits * MBp * c.n_q_heads * 2))) return rc;
   {
     const size_t tiles_h = (size_t)(H + 127) / 128;
     w->ssq_stride = round_up(std::max(MT, MBp), 16);
     const size_t st = (size_t)w->ssq_stride;
-    if ((rc = dalloc(&w->ssq_e, st)) || (rc = dalloc(&w->ssq_o, tiles_h * st)) || (rc = dalloc(&w->ssq_d, tiles_h * st)))
+    if ((rc = m.dev(&w->ssq_e, st)) || (rc = m.dev(&w->ssq_o, tiles_h * st)) || (rc = m.dev(&w->ssq_d, tiles_h * st)))
       return rc;
     const char* e = getenv("MQ_DECODE_CHAIN");
     w->chain = !(e && e[0] == '0');
@@ -132,57 +154,38 @@ static int worker_alloc(mq_worker* w) {
         set_last_error("MQ_TRACE: more launches per pass than trace slots");
         return MQ_ERR_INVAL;
       }
-      if ((rc = dalloc(&w->d_trace, (size_t)kTraceSlots * 4))) return rc;
+      if ((rc = m.dev(&w->d_trace, (size_t)kTraceSlots * 4))) return rc;
       CUDA_TRY(cudaMemsetAsync(w->d_trace, 0xFF, (size_t)kTraceSlots * 4 * 8, w->stream));
     }
   }
-  if ((rc = dalloc(&w->d_split_counter, (size_t)MBp * c.n_kv_heads))) return rc;
+  if ((rc = m.dev(&w->d_split_counter, (size_t)MBp * c.n_kv_heads))) return rc;
   CUDA_TRY(cudaMemsetAsync(w->d_split_counter, 0, (size_t)MBp * c.n_kv_heads * 4, w->stream));
-  if ((rc = dalloc(&w->inv_freq, D / 2))) return rc;
-  if ((rc = dalloc(&w->d_tok, MT))) return rc;
-  if ((rc = dalloc(&w->d_pos_tok, MT))) return rc;
-  if ((rc = dalloc(&w->d_slot_tok, MT))) return rc;
-  if ((rc = dalloc(&w->d_last_idx, MBp))) return rc;
-  if ((rc = dalloc(&w->d_dst_slot, MBp))) return rc;
-  if ((rc = dalloc(&w->d_tiles, MT + MB))) return rc;
-  if ((rc = dalloc(&w->d_cur_token, MBp))) return rc;
-  if ((rc = dalloc(&w->d_pos, MBp))) return rc;
-  if ((rc = dalloc(&w->d_active, MBp))) return rc;
-  if ((rc = dalloc(&w->d_temp, MBp)) || (rc = dalloc(&w->d_topp, MBp)) || (rc = dalloc(&w->d_topk, MBp)) ||
-      (rc = dalloc(&w->d_seed, MBp)))
-    return rc;
-  CUDA_TRY(cudaMemsetAsync(w->d_temp, 0, MBp * 4, w->stream));
-  CUDA_TRY(cudaMemsetAsync(w->d_topp, 0, MBp * 4, w->stream));
-  CUDA_TRY(cudaMemsetAsync(w->d_topk, 0, MBp * 4, w->stream));
-  CUDA_TRY(cudaMemsetAsync(w->d_seed, 0, MBp * 8, w->stream));
-  if ((rc = dalloc(&w->d_lp_top, MBp)) || (rc = dalloc(&w->d_lp_ring, (size_t)kRing * MBp))) return rc;
-  CUDA_TRY(cudaMemsetAsync(w->d_lp_top, 0xFF, MBp * 4, w->stream));  // -1: off
-  if ((rc = dalloc(&w->d_identity, MBp))) return rc;
-  if ((rc = dalloc(&w->d_block_table, (size_t)MBp * w->max_pages))) return rc;
-  if ((rc = dalloc(&w->d_out_ring, (size_t)kRing * MBp))) return rc;
+  if ((rc = m.dev(&w->inv_freq, D / 2))) return rc;
+  if ((rc = m.dev(&w->d_tok, MT))) return rc;
+  if ((rc = m.dev(&w->d_pos_tok, MT))) return rc;
+  if ((rc = m.dev(&w->d_slot_tok, MT))) return rc;
+  if ((rc = m.dev(&w->d_last_idx, MBp))) return rc;
+  if ((rc = m.dev(&w->d_dst_slot, MBp))) return rc;
+  if ((rc = m.dev(&w->d_tiles, MT + MB))) return rc;
+  if ((rc = m.dev(&w->d_cur_token, MBp))) return rc;
   CUDA_TRY(cudaMemsetAsync(w->d_cur_token, 0, MBp * 4, w->stream));
-  CUDA_TRY(cudaMemsetAsync(w->d_pos, 0, MBp * 4, w->stream));
-  CUDA_TRY(cudaMemsetAsync(w->d_active, 0, MBp * 4, w->stream));
-  CUDA_TRY(cudaMemsetAsync(w->d_block_table, 0, (size_t)MBp * w->max_pages * 4, w->stream));  // scratch page 0
+  if ((rc = m.dev(&w->d_identity, MBp))) return rc;
+  if ((rc = m.dev(&w->d_out_ring, (size_t)kRing * MBp)) || (rc = m.dev(&w->d_lp_ring, (size_t)kRing * MBp))) return rc;
+  if ((rc = m.host(&w->h_out_ring, (size_t)kRing * MBp)) || (rc = m.host(&w->h_lp_ring, (size_t)kRing * MBp))) return rc;
 
-  // pinned host
-  CUDA_TRY(cudaMallocHost((void**)&w->h_pos, MBp * 4));
-  CUDA_TRY(cudaMallocHost((void**)&w->h_active, MBp * 4));
-  CUDA_TRY(cudaMallocHost((void**)&w->h_temp, MBp * 4));
-  CUDA_TRY(cudaMallocHost((void**)&w->h_topp, MBp * 4));
-  CUDA_TRY(cudaMallocHost((void**)&w->h_topk, MBp * 4));
-  CUDA_TRY(cudaMallocHost((void**)&w->h_seed, MBp * 8));
-  memset(w->h_temp, 0, MBp * 4); memset(w->h_topp, 0, MBp * 4); memset(w->h_topk, 0, MBp * 4); memset(w->h_seed, 0, MBp * 8);
-  CUDA_TRY(cudaMallocHost((void**)&w->h_lp_top, MBp * 4));
-  memset(w->h_lp_top, 0xFF, MBp * 4);
-  CUDA_TRY(cudaMallocHost((void**)&w->h_lp_ring, (size_t)kRing * MBp * sizeof(LogprobRec)));
-  CUDA_TRY(cudaMallocHost((void**)&w->h_block_table, (size_t)MBp * w->max_pages * 4));
-  memset(w->h_pos, 0, MBp * 4);
-  memset(w->h_active, 0, MBp * 4);
-  memset(w->h_block_table, 0, (size_t)MBp * w->max_pages * 4);
-  w->stage_ints = (size_t)3 * MT + 4 * (size_t)(MT + MB) + 11 * (size_t)MBp + (size_t)MBp * w->max_pages + 64;
-  CUDA_TRY(cudaMallocHost((void**)&w->h_stage, w->stage_ints * 4 * kStageSlots));
-  CUDA_TRY(cudaMallocHost((void**)&w->h_out_ring, (size_t)kRing * MBp * 4));
+  // slot table (MBp % 16 == 0 keeps every section 64-byte aligned); every slot starts idle on scratch page 0
+  w->slot_bytes = (size_t)MBp * (6 * 4 + 8 + (size_t)w->max_pages * 4);
+  if ((rc = m.dev(&w->d_slots, w->slot_bytes)) || (rc = m.host(&w->h_slots, w->slot_bytes))) return rc;
+  carve(carve(w->h_slots, MBp, &w->h_pos, &w->h_active, &w->h_temp, &w->h_topk, &w->h_topp, &w->h_seed, &w->h_lp_top),
+        (size_t)MBp * w->max_pages, &w->h_block_table);
+  carve(carve(w->d_slots, MBp, &w->d_pos, &w->d_active, &w->d_temp, &w->d_topk, &w->d_topp, &w->d_seed, &w->d_lp_top),
+        (size_t)MBp * w->max_pages, &w->d_block_table);
+  memset(w->h_slots, 0, w->slot_bytes);
+  for (int s = 0; s < MBp; ++s) set_slot_sampling(w, s, SamplingParams{});
+  CUDA_TRY(cudaMemcpyAsync(w->d_slots, w->h_slots, w->slot_bytes, cudaMemcpyHostToDevice, w->stream));
+  // one staging area holds either a prefill pass's token metadata (launch_prefill) or a copy of the slot table
+  w->stage_ints = std::max((size_t)3 * MT + 4 * (size_t)(MT + MB) + 2 * (size_t)MBp, w->slot_bytes / 4);
+  if ((rc = m.host(&w->h_stage, w->stage_ints * kStageSlots))) return rc;
   w->stage_ev.resize(kStageSlots);
   for (auto& e : w->stage_ev) CUDA_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
 
@@ -197,7 +200,7 @@ static int worker_alloc(mq_worker* w) {
   // decode attention read exactly the values the table-less kernel would compute
   {
     const size_t n_pos = (size_t)w->max_pages * kPageSize;
-    if ((rc = dalloc(&w->rope_table, n_pos * (D / 2)))) return rc;
+    if ((rc = m.dev(&w->rope_table, n_pos * (D / 2)))) return rc;
     launch_rope_table(w->stream, w->rope_table, w->inv_freq, (int)n_pos, D / 2);
   }
   CUDA_TRY(cudaStreamSynchronize(w->stream));
@@ -522,36 +525,23 @@ static cudaEvent_t ev_get(mq_worker* w) {
   return e;
 }
 
-// upload the host mirrors of the slot table (pos / active / block table) when they changed
+// upload the slot table's host mirror when it changed (through a staging area: the mirror keeps changing while the copy
+// is still queued)
 static void upload_slots(mq_worker* w) {
   if (!w->slots_dirty) return;
-  const int MBp = round_up(w->MB, 16);
   int ss;
   int* st = stage_acquire(w, &ss);
-  int* s_pos = st;
-  int* s_act = st + MBp;
-  int* s_bt = st + 2 * MBp;
-  // temperature | top_k | top_p | seed (2 ints each) | top_logprobs
-  int* s_samp = s_bt + (size_t)MBp * w->max_pages;
-  int* s_lp = s_samp + 5 * MBp + (MBp & 1);
-  memcpy(s_samp, w->h_temp, MBp * 4);
-  memcpy(s_samp + MBp, w->h_topk, MBp * 4);
-  memcpy(s_samp + 2 * MBp, w->h_topp, MBp * 4);
-  memcpy(s_samp + 3 * MBp + (MBp & 1), w->h_seed, MBp * 8);
-  memcpy(s_lp, w->h_lp_top, MBp * 4);
-  cudaMemcpyAsync(w->d_temp, s_samp, MBp * 4, cudaMemcpyHostToDevice, w->stream);
-  cudaMemcpyAsync(w->d_topk, s_samp + MBp, MBp * 4, cudaMemcpyHostToDevice, w->stream);
-  cudaMemcpyAsync(w->d_topp, s_samp + 2 * MBp, MBp * 4, cudaMemcpyHostToDevice, w->stream);
-  cudaMemcpyAsync(w->d_seed, s_samp + 3 * MBp + (MBp & 1), MBp * 8, cudaMemcpyHostToDevice, w->stream);
-  cudaMemcpyAsync(w->d_lp_top, s_lp, MBp * 4, cudaMemcpyHostToDevice, w->stream);
-  memcpy(s_pos, w->h_pos, MBp * 4);
-  memcpy(s_act, w->h_active, MBp * 4);
-  memcpy(s_bt, w->h_block_table, (size_t)MBp * w->max_pages * 4);
-  cudaMemcpyAsync(w->d_pos, s_pos, MBp * 4, cudaMemcpyHostToDevice, w->stream);
-  cudaMemcpyAsync(w->d_active, s_act, MBp * 4, cudaMemcpyHostToDevice, w->stream);
-  cudaMemcpyAsync(w->d_block_table, s_bt, (size_t)MBp * w->max_pages * 4, cudaMemcpyHostToDevice, w->stream);
+  memcpy(st, w->h_slots, w->slot_bytes);
+  cudaMemcpyAsync(w->d_slots, st, w->slot_bytes, cudaMemcpyHostToDevice, w->stream);
   stage_release(w, ss);
   w->slots_dirty = false;
+}
+
+// sampler controls of a pass: the slot table's sampling sections, the per-slot RNG counter (nullptr: position 0) and the
+// pass's row of the log-probability ring
+static SampleCtl sample_ctl(mq_worker* w, const int* counter, int ring) {
+  return SampleCtl{w->d_temp, w->d_topk, w->d_topp, w->d_seed, counter, w->d_lp_top,
+                   w->d_lp_ring + (size_t)ring * round_up(w->MB, 16)};
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -569,7 +559,7 @@ static void free_slot(mq_worker* w, mq_req* r) {
   w->slot_req[s] = nullptr;
   w->h_active[s] = 0;
   w->h_pos[s] = 0;
-  w->h_lp_top[s] = -1;
+  set_slot_sampling(w, s, SamplingParams{});
   for (int i = 0; i < w->max_pages; ++i) w->h_block_table[(size_t)s * w->max_pages + i] = 0;  // scratch page
   w->slots_dirty = true;
   r->slot = -1;
@@ -590,7 +580,7 @@ static void finish_req(mq_worker* w, mq_req* r, int rc, const char* msg) {
   if (rc == 0) {
     send_status(r);
     std::string tail = frame_final(r->rq.endpoint, r->rq.stream, w->cfg.model_name, r->agg, (int)r->prompt.size(),
-                                   r->n_emitted, r->stopped, r->top_logprobs >= 0 ? &r->agg_lp : nullptr);
+                                   r->n_emitted, r->stopped, r->sp.top_logprobs >= 0 ? &r->agg_lp : nullptr);
     if (!tail.empty() && r->cb.on_chunk) r->cb.on_chunk(r->user, (const uint8_t*)tail.data(), tail.size());
   }
   if (r->cb.on_done) r->cb.on_done(r->user, rc, msg ? msg : "");
@@ -610,11 +600,11 @@ static void emit_token(mq_worker* w, mq_req* r, int tok, const LogprobRec* rec) 
   if (r->n_emitted == 0) r->t_first = Clock::now();
   r->n_emitted++;
   send_status(r);
-  if (r->top_logprobs >= 0) {
+  if (r->sp.top_logprobs >= 0) {
     TokenLogprobs e;
     e.id = tok;
     e.logprob = rec->logprob;
-    for (int j = 0; j < r->top_logprobs; ++j) e.top.push_back({rec->id[j], rec->lp[j]});
+    for (int j = 0; j < r->sp.top_logprobs; ++j) e.top.push_back({rec->id[j], rec->lp[j]});
     std::string s;
     if (r->rq.endpoint == MQ_EP_RAW_TOKENS) append_raw_record(r->rq.stream ? &s : &r->agg, e);
     else if (r->rq.stream) s = frame_token(r->rq.endpoint, w->cfg.model_name, tok, &e, r->text_len);
@@ -714,13 +704,12 @@ static int launch_prefill(mq_worker* w, std::vector<PrefillItem>& items) {
     const LaunchCfg lc{w->stream, c.use_pdl != 0};
     // first generated token of each finished prompt: RNG position 0 (decode steps use the token position >= 1)
     launch_sample(lc, w->logits, n_last, c.vocab, c.vocab, w->d_out_ring + (size_t)ring * MBp, w->d_dst_slot,
-                  w->d_cur_token, nullptr, nullptr,
-                  SampleCtl{w->d_temp, w->d_topk, w->d_topp, w->d_seed, nullptr, w->d_lp_top, w->d_lp_ring + (size_t)ring * MBp});
+                  w->d_cur_token, nullptr, nullptr, sample_ctl(w, nullptr, ring));
     ++nl;
     cudaMemcpyAsync(w->h_out_ring + (size_t)ring * MBp, w->d_out_ring + (size_t)ring * MBp, n_last * 4,
                     cudaMemcpyDeviceToHost, w->stream);
     bool want_lp = false;
-    for (auto& it : items) want_lp |= it.completes && it.r->top_logprobs >= 0;
+    for (auto& it : items) want_lp |= it.completes && it.r->sp.top_logprobs >= 0;
     if (want_lp)
       cudaMemcpyAsync(w->h_lp_ring + (size_t)ring * MBp, w->d_lp_ring + (size_t)ring * MBp, n_last * sizeof(LogprobRec),
                       cudaMemcpyDeviceToHost, w->stream);
@@ -773,8 +762,7 @@ static int decode_body(mq_worker* w, int Bcap, int n_splits, int attn_stages, in
   // NOTE: the ring slot is baked into a captured graph, so graphs write to a fixed staging row (ring 0 of the
   // graph area) and the copy-out below moves it into the real ring slot.
   launch_sample(lc, w->logits, Bcap, c.vocab, c.vocab, w->d_out_ring + (size_t)ring * MBp, nullptr, w->d_cur_token,
-                w->d_pos, w->d_active,
-                SampleCtl{w->d_temp, w->d_topk, w->d_topp, w->d_seed, w->d_pos, w->d_lp_top, w->d_lp_ring + (size_t)ring * MBp});
+                w->d_pos, w->d_active, sample_ctl(w, w->d_pos, ring));
   *nl += 1;
   return MQ_OK;
 }
@@ -787,7 +775,7 @@ static int launch_decode(mq_worker* w) {
   for (int s = 0; s < w->MB; ++s)
     if (w->h_active[s]) {
       hi = s;
-      want_lp |= w->slot_req[s]->top_logprobs >= 0;
+      want_lp |= w->slot_req[s]->sp.top_logprobs >= 0;
       ++n_active;
       max_ctx = std::max(max_ctx, w->h_pos[s] + 1);
       kv_tokens += w->h_pos[s] + 1;
@@ -980,8 +968,7 @@ static bool admit(mq_worker* w, mq_req* r) {
   }
   w->h_pos[slot] = 0;
   w->h_active[slot] = 0;
-  w->h_temp[slot] = r->temperature; w->h_topk[slot] = r->top_k; w->h_topp[slot] = r->top_p; w->h_seed[slot] = r->seed;
-  w->h_lp_top[slot] = r->top_logprobs;
+  set_slot_sampling(w, slot, r->sp);
   w->slots_dirty = true;
   return true;
 }
@@ -1274,15 +1261,8 @@ void mq_worker_close(mq_worker* w) {
   }
   if (w->stream) cudaStreamSynchronize(w->stream);
   for (auto& kv : w->graphs) cudaGraphExecDestroy(kv.second);
-  for (auto& kv : w->tensors) cudaFree(kv.second.ptr);
   streamk_workspace_free(&w->sk_ws);
-  void* bufs[] = {w->k_cache, w->v_cache, w->h, w->x, w->q, w->attn, w->act, w->x_last, w->qkv_part, w->proj_part,
-                  w->logits, w->part_o, w->part_ml, w->inv_freq, w->d_tok, w->d_pos_tok, w->d_slot_tok, w->d_last_idx,
-                  w->d_dst_slot, w->d_tiles, w->d_cur_token, w->d_pos, w->d_active, w->d_block_table, w->d_identity,
-                  w->d_out_ring, w->d_split_counter, w->ssq_e, w->ssq_o, w->ssq_d, w->d_lp_top, w->d_lp_ring};
-  for (void* b : bufs) if (b) cudaFree(b);
-  void* pinned[] = {w->h_pos, w->h_active, w->h_block_table, w->h_stage, w->h_out_ring, w->h_lp_top, w->h_lp_ring};
-  for (void* b : pinned) if (b) cudaFreeHost(b);
+  w->allocs.free_all();
   for (auto e : w->stage_ev) cudaEventDestroy(e);
   for (auto e : w->ev_pool) cudaEventDestroy(e);
   if (w->stream) cudaStreamDestroy(w->stream);
@@ -1402,11 +1382,11 @@ int mq_submit(mq_worker* w, const mq_request* rq, const mq_callbacks* cb, void* 
   if (r->prompt.empty()) r->prompt.push_back(0);
   for (int32_t& t : r->prompt) if (t < 0 || t >= w->cfg.vocab) t = 0;
   r->rq.body = nullptr; r->rq.prompt_tokens = nullptr;
-  if (pb.has_stream && rq->stream < 0) r->rq.stream = pb.stream ? 1 : 0;
+  apply_body(pb, &r->rq);  // a no-op when there was no JSON body to parse; from here on only r->rq is read
   if (r->rq.stream < 0) r->rq.stream = 1;
   // generation length: validated BEFORE any arithmetic with the prompt length ("num_predict": 2147483647 used to wrap
   // prompt + max_new negative, pass both checks below and die in vector::resize on the worker thread)
-  long long want = rq->max_new_tokens > 0 ? rq->max_new_tokens : (pb.num_predict > 0 ? pb.num_predict : 128);
+  long long want = r->rq.max_new_tokens > 0 ? r->rq.max_new_tokens : 128;
   if (want > (long long)w->cfg.max_seq - (long long)r->prompt.size()) {
     const int n = (int)r->prompt.size();
     delete r;
@@ -1414,23 +1394,21 @@ int mq_submit(mq_worker* w, const mq_request* rq, const mq_callbacks* cb, void* 
     return MQ_ERR_INVAL;
   }
   r->max_new = (int)want;
-  // sampling: body options win over the struct fields; everything unset = greedy (what BASELINE measures)
-  r->temperature = pb.has_temperature ? (float)pb.temperature : rq->temperature;
-  r->top_k = pb.has_top_k ? (int)std::min<long long>(pb.top_k, 1 << 30) : rq->top_k;
-  r->top_p = pb.has_top_p ? (float)pb.top_p : rq->top_p;
-  r->seed = pb.has_seed ? pb.seed : rq->seed;
-  if (pb.has_logprobs ? pb.logprobs : rq->logprobs != 0)
-    r->top_logprobs = pb.has_top_logprobs ? pb.top_logprobs : std::max(0, std::min<int>(rq->top_logprobs, MQ_TOP_LOGPROBS_MAX));
-  if (!(r->temperature == r->temperature)) r->temperature = 0.f;  // NaN from a C-ABI caller: greedy
-  if (!(r->top_p == r->top_p)) r->top_p = 0.f;
+  // sampling: everything unset = greedy (what BASELINE measures); NaN from a C-ABI caller is greedy / off too
+  SamplingParams& sp = r->sp;
+  sp.temperature = r->rq.temperature == r->rq.temperature ? r->rq.temperature : 0.f;
+  sp.top_k = r->rq.top_k;
+  sp.top_p = r->rq.top_p == r->rq.top_p ? r->rq.top_p : 0.f;
+  sp.seed = r->rq.seed;
+  if (r->rq.logprobs) sp.top_logprobs = std::max(0, std::min<int>(r->rq.top_logprobs, MQ_TOP_LOGPROBS_MAX));
   if (((long long)r->prompt.size() + r->max_new + kPageSize - 1) / kPageSize > w->n_pages - 1) {
     delete r;
     set_last_error("request needs more KV pages than the worker owns (%d)", w->n_pages - 1);
     return MQ_ERR_NOMEM;
   }
-  if (rq->timeout_ms) {
+  if (r->rq.timeout_ms) {
     r->has_deadline = true;
-    r->deadline = r->t_submit + std::chrono::milliseconds(rq->timeout_ms);
+    r->deadline = r->t_submit + std::chrono::milliseconds(r->rq.timeout_ms);
   }
   if (out) *out = r; else r->refs.store(1);
   {

@@ -25,6 +25,25 @@ struct DevTensor {
   size_t bytes = 0;
 };
 
+// Owner of every device and pinned host allocation of a worker or an encoder: each one is recorded when it is made and
+// free_all releases them together, so a close after a partial setup frees exactly what setup got.
+struct Allocations {
+  std::vector<void*> dev_ptrs, host_ptrs;
+  int alloc(void** p, size_t bytes, bool pinned_host);  // MQ_ERR_NOMEM (with the error text set) on failure
+  template <typename T> int dev(T** p, size_t n) { return alloc(reinterpret_cast<void**>(p), n * sizeof(T), false); }
+  template <typename T> int host(T** p, size_t n) { return alloc(reinterpret_cast<void**>(p), n * sizeof(T), true); }
+  void free_all();
+};
+
+// Per-request sampling settings, also one entry per slot in the worker's slot table
+struct SamplingParams {
+  float temperature = 0.f;  // <= 0: greedy
+  int top_k = 0;            // <= 0: off
+  float top_p = 0.f;        // <= 0 or >= 1: off
+  unsigned long long seed = 0;
+  int top_logprobs = -1;  // -1: no logprobs; 0..MQ_TOP_LOGPROBS_MAX: a record per relayed token with that many alternatives
+};
+
 struct LayerWeights {
   __nv_bfloat16 *attn_norm, *wqkv, *bqkv, *wo, *mlp_norm, *w_gate_up, *w_down;
 };
@@ -61,10 +80,7 @@ struct mq_req {
   int n_sched = 0;       // generated tokens scheduled on the GPU so far
   int n_emitted = 0;     // generated tokens delivered to the callback
   int max_new = 0;
-  float temperature = 0.f, top_p = 0.f;  // sampling controls (0 = greedy / off)
-  int top_k = 0;
-  unsigned long long seed = 0;
-  int top_logprobs = -1;  // -1: no logprobs; 0..MQ_TOP_LOGPROBS_MAX: a record per relayed token with that many alternatives
+  mq::SamplingParams sp;
   size_t text_len = 0;    // characters relayed so far (/v1/completions text_offset)
   std::vector<mq::TokenLogprobs> agg_lp;  // stream=0 with logprobs: every relayed token's entry
   std::atomic<bool> cancel{false};
@@ -89,6 +105,7 @@ struct mq_worker {
   cudaStream_t stream = nullptr;
   int qkv_dim = 0, max_pages = 0, n_pages = 0, MT = 0, MB = 0;
   double p_mm_bytes = 0, kv_bytes_per_tok = 0;
+  mq::Allocations allocs;  // owns every buffer below (weights included) except the stream-K workspace
 
   // weights
   std::map<std::string, mq::DevTensor> tensors;
@@ -106,8 +123,14 @@ struct mq_worker {
   // metadata (device)
   int *d_tok = nullptr, *d_pos_tok = nullptr, *d_slot_tok = nullptr, *d_last_idx = nullptr, *d_dst_slot = nullptr;
   int4* d_tiles = nullptr;
-  int *d_cur_token = nullptr, *d_pos = nullptr, *d_active = nullptr, *d_block_table = nullptr, *d_identity = nullptr;
-  // per-slot sampling controls (device) + pinned host mirrors, uploaded with the slot table
+  int *d_cur_token = nullptr, *d_identity = nullptr;
+  // slot table: a pinned host mirror (h_slots) and its device copy (d_slots) with one layout, sections of MBp entries
+  // pos | active | temperature | top_k | top_p | seed | top_logprobs | block_table, uploaded whole when it changed.
+  // The d_* / h_* pointers below are views into the two blocks (captured graphs read the d_* views).
+  uint8_t *d_slots = nullptr, *h_slots = nullptr;
+  size_t slot_bytes = 0;
+  int *d_pos = nullptr, *d_active = nullptr, *d_block_table = nullptr;
+  int *h_pos = nullptr, *h_active = nullptr, *h_block_table = nullptr;
   float *d_temp = nullptr, *d_topp = nullptr, *h_temp = nullptr, *h_topp = nullptr;
   int *d_topk = nullptr, *h_topk = nullptr;
   unsigned long long *d_seed = nullptr, *h_seed = nullptr;
@@ -125,8 +148,7 @@ struct mq_worker {
   std::vector<CUtensorMap> tm_k, tm_v;
   bool chain = true;         // MQ_DECODE_CHAIN=0: the round-1 plane-based decode path (A/B and parity cross-check)
   unsigned long long* d_trace = nullptr;  // MQ_TRACE=1: [kTraceSlots][4] %globaltimer stamps of the latest pass
-  // pinned host mirrors / staging
-  int *h_pos = nullptr, *h_active = nullptr, *h_block_table = nullptr;
+  // pinned host staging
   int* h_stage = nullptr;     // ring of staging areas for metadata uploads
   int* h_out_ring = nullptr;  // [kRing][MB]
   mq::LogprobRec* h_lp_ring = nullptr;  // [kRing][MB]

@@ -291,6 +291,17 @@ bool parse_body(const std::string& body, int endpoint, ParsedBody* out) {
   return j.p == j.e;  // nothing but whitespace after the object
 }
 
+void apply_body(const ParsedBody& pb, mq_request* rq) {
+  if (pb.has_stream && rq->stream < 0) rq->stream = pb.stream ? 1 : 0;
+  if (rq->max_new_tokens <= 0 && pb.num_predict > 0) rq->max_new_tokens = pb.num_predict;
+  if (pb.has_temperature) rq->temperature = (float)pb.temperature;
+  if (pb.has_top_k) rq->top_k = (int32_t)pb.top_k;  // parse_body clamped it to 0..2^30
+  if (pb.has_top_p) rq->top_p = (float)pb.top_p;
+  if (pb.has_seed) rq->seed = pb.seed;
+  if (pb.has_logprobs) rq->logprobs = pb.logprobs ? 1 : 0;
+  if (pb.has_top_logprobs) rq->top_logprobs = (int16_t)pb.top_logprobs;
+}
+
 // deterministic byte-level tokenizer: random-init weights have no vocabulary (SURVEY.md 7)
 std::vector<int32_t> byte_tokenize(const std::string& text, int vocab) {
   std::vector<int32_t> t;

@@ -3,6 +3,7 @@
 // OpenAI wire shapes seen in the reference's own client script (test_dispatcher.sh:37-39,69,93) and README.
 // Parity here is UNPINNED by the reference (SURVEY.md 7 "hard parts").
 #pragma once
+#include "../../include/ollamamq_b200.h"
 #include <cstdint>
 #include <string>
 #include <utility>
@@ -37,6 +38,9 @@ struct TokenLogprobs {
 };
 
 bool parse_body(const std::string& body, int endpoint, ParsedBody* out);
+// Folds a parsed body into the request: "stream" when the request left it to the body (< 0), the body's num_predict
+// when max_new_tokens is unset (<= 0), and every sampling / logprobs option the body sets, over the struct's value.
+void apply_body(const ParsedBody& pb, mq_request* rq);
 std::vector<int32_t> byte_tokenize(const std::string& text, int vocab);
 std::string token_text(int tok);
 const char* content_type_for(int endpoint, int stream);
